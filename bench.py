@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (libfsgpu.so on N B200s)
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: the reference's CPU renderer on host cores
     python bench.py --workload NAME                          # another BASELINE config as the headline (see WORKLOADS)
+    python bench.py --dump-outputs DIR ...                   # also write the last timed step's frame to DIR/*.npy
 
 Headline workload (config.workload): View #14 (north_star's target view: 6,632-digit coordinates, zoom 4.7e6516,
 maxIter 2,147,483,646), GpuHDRx32PerturbedLAv2, 3840x2160, AA 1, u32 iterations (BASELINE.json configs[3]).  The
@@ -335,6 +336,26 @@ def run_reference_arm(args, rank):
     print(json.dumps(line), flush=True)
 
 
+DUMP_SEED = 20240607
+DUMP_SAMPLE_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, iters, red, width, height):
+    """What the timed render hands its caller, as float64 .npy files: the reduction [Min, Max, Sum // 2^32, Sum % 2^32],
+    every row's and column's sum of the iteration buffer, and the whole rows of a fixed, seeded sample of the frame (about
+    32 MB) with their row numbers.  All exact: counts are below 2^32 and a row or column has fewer than 2^21 of them."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    frame = iters[:height, :width].astype(np.float64)
+    n_rows = min(height, max(1, DUMP_SAMPLE_BYTES // (8 * width)))
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(height, size=n_rows, replace=False))
+    arrays = {"reduction": np.array([red["Min"], red["Max"], red["Sum"] >> 32, red["Sum"] & 0xFFFFFFFF], dtype=np.float64),
+              "row_sums": frame.sum(axis=1), "column_sums": frame.sum(axis=0),
+              "sample_rows": rows.astype(np.float64), "iterations_sample_rows": frame[rows]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def metric_name(wl):
     return f"pixel-iters/sec (device-timed) for {wl.where.replace('view', 'View ')} perturb+LA" if wl.traits.family != "direct" \
         else f"pixel-iters/sec (device-timed) for {wl.where} direct escape time"
@@ -351,7 +372,11 @@ def main():
     ap.add_argument("--configs", default=None, help="comma-separated workload names for the `configs` array")
     ap.add_argument("--workload", default=None, choices=sorted(WORKLOADS), help="headline workload (default: View 14 HDRx32 LAv2)")
     ap.add_argument("--view", type=int, default=None, choices=[5, 14], help="shorthand: --view 5 = --workload view5_hdr32_lav2")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the frame the last timed step rendered to DIR/<name>.npy (float64; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.workload is None:
         args.workload = "view5_hdr32_lav2" if args.view == 5 else HEADLINE
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
@@ -474,6 +499,18 @@ def main():
     barrier()
     wall_s = time.time() - t_wall0
     launches_timed = r.KernelLaunchCount() - launches0 - args.warmup
+    if args.dump_outputs:
+        # untimed: the frame of the last timed step, assembled on rank 0 (disjoint rows, so SUM == gather)
+        rc, last_iters, _, last_red = r.RenderCurrent(n_iter)
+        assert rc == 0
+        if world > 1:
+            dev = torch.from_numpy(last_iters.view(np.int32)).cuda()
+            dist.reduce(dev, dst=0, op=dist.ReduceOp.SUM)
+            last_iters = dev.cpu().numpy().view(np.uint32)
+            frame = last_iters[:height, :width]
+            last_red = {"Min": int(frame.min()), "Max": int(frame.max()), "Sum": int(frame.astype(np.int64).sum())}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, last_iters, last_red, width, height)
     # executed-step count for the roofline: one extra, untimed launch of the counting variant of the kernel
     r.EnableStepCounter(True)
     step_resident()

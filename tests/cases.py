@@ -158,6 +158,49 @@ def inputs_crc(coords, orbit, table):
     return crc
 
 
+def sha256_of(a):
+    import hashlib
+    import numpy as np
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def la_digest(la):
+    """Sizes and SHA-256 digests of an LA table (LAInfoDeep[] with its indeterminate padding cleared, the LAStageCount
+    stage records, the ATInfo bytes), as stored in tests/golden/tables.json."""
+    import ctypes as C
+    import numpy as np
+    las = la.las_numpy().copy()
+    if la.iter_bytes == 8:
+        las[:, 60:64] = 0   # LAInfoDeep<uint64_t, ...>: 4 padding bytes between MinMag (ends at 60) and LAi (at 64)
+    at = np.frombuffer((C.c_ubyte * la.at_bytes).from_address(la.descriptor().at), dtype=np.uint8)
+    return {"num_las": la.num_las, "stage_count": la.stage_count, "use_at": bool(la.use_at), "is_valid": bool(la.is_valid),
+            "las_elem_bytes": la.las_elem_bytes, "at_bytes": la.at_bytes, "las_sha256": sha256_of(las),
+            "stages_sha256": sha256_of(la.stages_numpy()[: la.stage_count]), "at_sha256": sha256_of(at)}
+
+
+def bla_digest(bl):
+    """Level count, LM2 and the SHA-256 of every level of a BLA table, as stored in tests/golden/tables.json."""
+    return {"num_levels": bl.num_levels, "lm2": bl.lm2,
+            "levels_sha256": [sha256_of(bl.level_numpy(lv)) for lv in range(bl.num_levels)]}
+
+
+def full_case_precision(name):
+    """iteration_precision of a full-size case: the N of a `_pN` name suffix, else 1."""
+    return int(name.split("_p")[1].split("_")[0]) if "_p" in name and name.split("_p")[1][0].isdigit() else 1
+
+
+def load_recorded(name):
+    """A recording of tests/golden/record_library_outputs.py: .json as a dict, .npz as a dict of arrays."""
+    import json
+    import os
+    import numpy as np
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name)
+    if name.endswith(".json"):
+        with open(path) as f:
+            return json.load(f)
+    return dict(np.load(path))
+
+
 def oracle_render(alg, w, h, coords, orbit, table, n, ib, precision=1, **kw):
     """CPU oracle for a case, or None when the oracle has no restatement of that variant."""
     import oracle_cpu

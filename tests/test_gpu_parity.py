@@ -99,7 +99,7 @@ def test_full_size_vs_reference_cuda_kernels(case):
     north_star asks for FP64/FP32 direct bit-exact and HDRx32/2x32/LA >= 99.9 % exact with |d iter| <= 1 elsewhere;
     every case here is held to bit-exactness (1.0) except the four-limb direct kernels (DESIGN.md section 2)."""
     name, view_id, w, h, alg, n_iter, ib, min_exact = case
-    prec = int(name.split("_p")[1].split("_")[0]) if "_p" in name and name.split("_p")[1][0].isdigit() else 1
+    prec = cases.full_case_precision(name)
     _, coords, orbit, la, n = cases.make_inputs(view_id, w, h, alg, n_iter, ib)
     got, _, red = cases.render(GPURenderer, w, h, alg, coords, orbit, la, n, ib, precision=prec)
     ref, _, ref_red = cases.render(ref_renderer.RefGPURenderer, w, h, alg, coords, orbit, la, n, ib, precision=prec)
@@ -440,8 +440,11 @@ EDGE_CASES = [
 ]
 
 
+EDGE_IDS = [f"v{c[0]}_{c[1]}x{c[2]}_{c[3].name}_{c[4]}" for c in EDGE_CASES]
+
+
 @pytest.mark.skipif(not ref_renderer.available(), reason="oracle/_ref (reference CUDA kernels) not built")
-@pytest.mark.parametrize("case", EDGE_CASES, ids=[f"v{c[0]}_{c[1]}x{c[2]}_{c[3].name}_{c[4]}" for c in EDGE_CASES])
+@pytest.mark.parametrize("case", EDGE_CASES, ids=EDGE_IDS)
 def test_edge_shapes_and_limits_vs_reference_kernels(case):
     """1x1 and ragged frames (not multiples of the 16x8 padding or of the 8x4 work tile), iteration limits of a
     few steps, both iteration widths: same buffers as the reference kernels, padding cells left cleared."""
