@@ -931,7 +931,9 @@ void CUDART_CB done_trampoline(void *p) {
 // ---- per-operation self-test (fs_selftest_numeric_op) -------------------------------------------------------------
 // One operation of the device numeric types on arrays of operands, evaluated with the functions the render kernels
 // call (fs_types.cuh, fs_df32.cuh, fs_qd.cuh).  tests/test_gpu_parity.py compares the results with the oracle's
-// restatement of the reference's HDRFloat / HDRFloatComplex / dblflt / dbldbl routines, bit for bit.
+// restatement of the reference's HDRFloat / HDRFloatComplex / dblflt / dbldbl routines, bit for bit; the Quad<F> ops
+// (60-67, 70-77) have no restatement and are compared with the host build of fs_qd.cuh and with exact arithmetic
+// (tests/test_exact_escape.py).
 namespace {
 struct SelfHf { float m; int32_t e; };
 struct SelfHc { float re, im; int32_t e; };
@@ -988,6 +990,14 @@ __global__ void numeric_op_kernel(uint32_t op, const void *a_, const void *b_, v
     case 30: static_cast<dd64 *>(out_)[i] = dd_add(qa[i], qb[i]); break;
     case 31: static_cast<dd64 *>(out_)[i] = dd_sub(qa[i], qb[i]); break;
     case 32: static_cast<dd64 *>(out_)[i] = dd_mul(qa[i], qb[i]); break;
+    case 60: case 61: case 62: case 63: case 64: case 65: case 66: case 67:
+        static_cast<Quad<double> *>(out_)[i] = quad_selftest_op<double>(op - 60, static_cast<const Quad<double> *>(a_)[i],
+                                                                        static_cast<const Quad<double> *>(b_)[i]);
+        break;
+    case 70: case 71: case 72: case 73: case 74: case 75: case 76: case 77:
+        static_cast<Quad<float> *>(out_)[i] = quad_selftest_op<float>(op - 70, static_cast<const Quad<float> *>(a_)[i],
+                                                                      static_cast<const Quad<float> *>(b_)[i]);
+        break;
     default: break;
     }
 }
@@ -998,6 +1008,8 @@ uint32_t numeric_op_elem_bytes(uint32_t op) {
     if (op >= 30 && op <= 32) return 16;
     if (op == 40) return 24;
     if (op >= 50 && op <= 56) return 16;
+    if (op >= 60 && op <= 67) return 32;
+    if (op >= 70 && op <= 77) return 16;
     return 0;
 }
 } // namespace

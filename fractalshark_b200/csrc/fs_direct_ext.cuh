@@ -81,49 +81,15 @@ struct Pixel2x64 {
 };
 
 // ---- Gpu4x32 / Gpu4x64 -------------------------------------------------------------------------------------------
-struct Pixel4x32 {
-    using Coord = Quad<float>;
+// the step loop is quad_escape_count (fs_qd.cuh), shared with the host build of the oracle
+template <class F> struct PixelQuad {
+    using Coord = Quad<F>;
     template <class IterT> FS_D static IterT run(const DirectExtArgs<Coord, IterT> &A, int X, int Y) {
-        using O = QuadOps<float>;
-        const Coord y0 = O::add(A.cy, O::mul(A.dy, O::make((float)Y, 0, 0, 0)));
-        const Coord x0 = O::add(A.cx, O::mul(A.dx, O::make((float)X, 0, 0, 0)));
-        const Coord four = O::make(4.0f, 0, 0, 0);
-        Coord x = O::make(0, 0, 0, 0), y = x;
-        Coord zr = O::sqr(x), zi = O::sqr(y);
-        IterT iter = 0;
-        while (O::le(O::add(zr, zi), four) && iter < A.n_iterations) {
-            y = O::mul(x, y);
-            y = O::mul_pwr2(y, 2.0f);
-            y = O::add(y, y0);
-            x = O::add(O::sub(zr, zi), x0);
-            zr = O::sqr(x);
-            zi = O::sqr(y);
-            iter++;
-        }
-        return iter;
+        return quad_escape_count<F, IterT>(A.cx, A.cy, A.dx, A.dy, X, Y, A.n_iterations);
     }
 };
-struct Pixel4x64 {
-    using Coord = Quad<double>;
-    template <class IterT> FS_D static IterT run(const DirectExtArgs<Coord, IterT> &A, int X, int Y) {
-        using O = QuadOps<double>;
-        const Coord y0 = O::add(A.cy, O::mul(A.dy, (double)Y));
-        const Coord x0 = O::add(A.cx, O::mul(A.dx, (double)X));
-        Coord x = O::make(0, 0, 0, 0), y = x;
-        Coord zr = O::mul(x, x), zi = O::mul(y, y);
-        IterT iter = 0;
-        while (O::le(O::add(zr, zi), 4.0) && iter < A.n_iterations) {
-            y = O::mul(x, y);
-            y = O::mul(y, 2.0);
-            y = O::add(y, y0);
-            x = O::add(O::sub(zr, zi), x0);
-            zr = O::mul(x, x);
-            zi = O::mul(y, y);
-            iter++;
-        }
-        return iter;
-    }
-};
+using Pixel4x32 = PixelQuad<float>;
+using Pixel4x64 = PixelQuad<double>;
 
 // ---- GpuHDRx32 (float+exponent over 2x32) ------------------------------------------------------------------------
 template <int P> struct PixelHdr2x32 {

@@ -14,13 +14,16 @@
 //             uses a Dekker split written with plain operators that its build leaves to the compiler's
 //             contraction; the two agree to the last limb's rounding (~2^-200 / ~2^-90 relative), far below
 //             what moves an escape count (tests/test_gpu_parity.py compares whole frames with the reference
-//             kernels).
+//             kernels; tests/test_exact_escape.py holds every operation to its error bound against exact
+//             rationals and the kernels' counts to exact arithmetic).
 #pragma once
 #include "fs_types.cuh"
 
 namespace fs {
 
 // ---- double-double -------------------------------------------------------------------------------------------
+// device only (__dadd_rn); QuadOps below is host-callable as well (oracle/lockstep_check.cpp builds it with g++)
+#ifdef __CUDACC__
 struct dd64 {
     double head, tail;
 };
@@ -64,6 +67,7 @@ FS_D dd64 dd_mul(dd64 a, dd64 b) { // mul_dbldbl  dbldbl.cuh:169-180 (sqr_dbldbl
     z.tail = __dadd_rn(__dadd_rn(th, -z.head), tt);
     return z;
 }
+#endif
 
 // ---- four-limb expansions --------------------------------------------------------------------------------------
 template <class F> struct Quad {
@@ -73,40 +77,40 @@ template <class F> struct QuadOps {
     static constexpr bool kBranchy = sizeof(F) == 8; // QuadDouble keeps the zero shortcuts, QuadFloat dropped them
     using Q = Quad<F>;
 
-    FS_D static Q make(F x, F y, F z, F w) { Q q; q.x = x; q.y = y; q.z = z; q.w = w; return q; }
+    FS_HD static Q make(F x, F y, F z, F w) { Q q; q.x = x; q.y = y; q.z = z; q.w = w; return q; }
     // fl(a+b), err; |a| >= |b|
-    FS_D static F quick_two_sum(F a, F b, F &err) {
+    FS_HD static F quick_two_sum(F a, F b, F &err) {
         if (kBranchy && b == F(0)) { err = F(0); return a + b; }
         const F s = a + b;
         err = b - (s - a);
         return s;
     }
-    FS_D static F two_sum(F a, F b, F &err) {
+    FS_HD static F two_sum(F a, F b, F &err) {
         if (kBranchy && (a == F(0) || b == F(0))) { err = F(0); return a + b; }
         const F s = a + b;
         const F bb = s - a;
         err = (a - (s - bb)) + (b - bb);
         return s;
     }
-    FS_D static F two_prod(F a, F b, F &err) {
+    FS_HD static F two_prod(F a, F b, F &err) {
         const F p = a * b;
         err = fma_(a, b, -p);
         return p;
     }
-    FS_D static void three_sum(F &a, F &b, F &c) {
+    FS_HD static void three_sum(F &a, F &b, F &c) {
         F t1, t2, t3;
         t1 = two_sum(a, b, t2);
         a = two_sum(c, t1, t3);
         b = two_sum(t2, t3, c);
     }
-    FS_D static void three_sum2(F &a, F &b, F &c) {
+    FS_HD static void three_sum2(F &a, F &b, F &c) {
         F t1, t2, t3;
         t1 = two_sum(a, b, t2);
         a = two_sum(c, t1, t3);
         b = t2 + t3;
     }
     // five limbs -> four
-    FS_D static void renorm(F &c0, F &c1, F &c2, F &c3, F &c4) {
+    FS_HD static void renorm(F &c0, F &c1, F &c2, F &c3, F &c4) {
         F s0, s1, s2 = F(0), s3 = F(0);
         s0 = quick_two_sum(c3, c4, c4);
         s0 = quick_two_sum(c2, s0, c3);
@@ -142,9 +146,9 @@ template <class F> struct QuadOps {
         }
         c0 = s0; c1 = s1; c2 = s2; c3 = s3;
     }
-    FS_D static Q neg(Q a) { return make(-a.x, -a.y, -a.z, -a.w); }
+    FS_HD static Q neg(Q a) { return make(-a.x, -a.y, -a.z, -a.w); }
     // sloppy_add  gqd_basic.cuh:177-225
-    FS_D static Q add(Q a, Q b) {
+    FS_HD static Q add(Q a, Q b) {
         F s0 = a.x + b.x, s1 = a.y + b.y, s2 = a.z + b.z, s3 = a.w + b.w;
         const F v0 = s0 - a.x, v1 = s1 - a.y, v2 = s2 - a.z, v3 = s3 - a.w;
         F u0 = s0 - v0, u1 = s1 - v1, u2 = s2 - v2, u3 = s3 - v3;
@@ -159,10 +163,10 @@ template <class F> struct QuadOps {
         renorm(s0, s1, s2, s3, t0);
         return make(s0, s1, s2, s3);
     }
-    FS_D static Q sub(Q a, Q b) { return add(a, neg(b)); }
-    FS_D static Q mul_pwr2(Q a, F b) { return make(a.x * b, a.y * b, a.z * b, a.w * b); }
+    FS_HD static Q sub(Q a, Q b) { return add(a, neg(b)); }
+    FS_HD static Q mul_pwr2(Q a, F b) { return make(a.x * b, a.y * b, a.z * b, a.w * b); }
     // quad * scalar  gqd_basic.cuh:267-292
-    FS_D static Q mul(Q a, F b) {
+    FS_HD static Q mul(Q a, F b) {
         F p0, p1, p2, p3, q0, q1, q2, s0, s1, s2, s3, s4;
         p0 = two_prod(a.x, b, q0);
         p1 = two_prod(a.y, b, q1);
@@ -178,7 +182,7 @@ template <class F> struct QuadOps {
         return make(s0, s1, s2, s3);
     }
     // sloppy_mul  gqd_basic.cuh:300-344
-    FS_D static Q mul(Q a, Q b) {
+    FS_HD static Q mul(Q a, Q b) {
         F p0, p1, p2, p3, p4, p5, q0, q1, q2, q3, q4, q5, t0, t1, s0, s1, s2;
         p0 = two_prod(a.x, b.x, q0);
         p1 = two_prod(a.x, b.y, q1);
@@ -199,7 +203,7 @@ template <class F> struct QuadOps {
         return make(p0, p1, s0, s1);
     }
     // sqr  gqd_basic.cuh:351-393
-    FS_D static Q sqr(Q a) {
+    FS_HD static Q sqr(Q a) {
         F p0, p1, p2, p3, p4, p5, q0, q1, q2, q3, s0, s1, t0, t1;
         p0 = two_prod(a.x, a.x, q0);
         p1 = two_prod(F(2) * a.x, a.y, q1);
@@ -226,10 +230,66 @@ template <class F> struct QuadOps {
         renorm(p0, p1, p2, p3, p4);
         return make(p0, p1, p2, p3);
     }
-    FS_D static bool le(Q a, Q b) { // operator<=(quad, quad)  gqd_basic.cuh:514-519
+    FS_HD static bool le(Q a, Q b) { // operator<=(quad, quad)  gqd_basic.cuh:514-519
         return a.x < b.x || (a.x == b.x && (a.y < b.y || (a.y == b.y && (a.z < b.z || (a.z == b.z && a.w <= b.w)))));
     }
-    FS_D static bool le(Q a, F b) { return a.x < b || (a.x == b && a.y <= F(0)); } // operator<=(quad, scalar) :531-533
+    FS_HD static bool le(Q a, F b) { return a.x < b || (a.x == b && a.y <= F(0)); } // operator<=(quad, scalar) :531-533
 };
+
+// The Quad<F> operations by number, for the per-operation self-test (fs_selftest_numeric_op 60-67 / 70-77) and its
+// host build: 0 add, 1 sub, 2 mul(q, q), 3 mul(q, b.x), 4 sqr(a), 5 mul_pwr2(a, b.x), 6 le(a, b), 7 le(a, b.x);
+// the comparisons return {1 or 0, 0, 0, 0}.
+template <class F> FS_HD Quad<F> quad_selftest_op(uint32_t k, Quad<F> a, Quad<F> b) {
+    using O = QuadOps<F>;
+    switch (k) {
+    case 0: return O::add(a, b);
+    case 1: return O::sub(a, b);
+    case 2: return O::mul(a, b);
+    case 3: return O::mul(a, b.x);
+    case 4: return O::sqr(a);
+    case 5: return O::mul_pwr2(a, b.x);
+    case 6: return O::make(O::le(a, b) ? F(1) : F(0), 0, 0, 0);
+    default: return O::make(O::le(a, b.x) ? F(1) : F(0), 0, 0, 0);
+    }
+}
+
+// The escape-time loop of the four-limb direct kernels (mandel_4x_float / mandel_4x_double, LowPrecisionKernels.cuh:5-144)
+// for the kernel's own pixel (X, Y), Y already flipped.  One iteration per bailout test, non-strict bailout on the
+// rounded quad sum, no n_iterations - (P-1).  The float flavour builds x0 with quad * quad and compares with a quad 4,
+// the double flavour with quad * scalar and a scalar 4, as the reference does.  Host-callable: oracle/lockstep_check.cpp
+// runs this very loop on the CPU.
+template <class F, class IterT>
+FS_HD IterT quad_escape_count(Quad<F> cx, Quad<F> cy, Quad<F> dx, Quad<F> dy, int X, int Y, IterT n_iterations) {
+    using O = QuadOps<F>;
+    using Q = Quad<F>;
+    Q x0, y0;
+    if constexpr (sizeof(F) == 4) {
+        y0 = O::add(cy, O::mul(dy, O::make((F)Y, 0, 0, 0)));
+        x0 = O::add(cx, O::mul(dx, O::make((F)X, 0, 0, 0)));
+    } else {
+        y0 = O::add(cy, O::mul(dy, (F)Y));
+        x0 = O::add(cx, O::mul(dx, (F)X));
+    }
+    Q x = O::make(0, 0, 0, 0), y = x;
+    Q zr, zi;
+    if constexpr (sizeof(F) == 4) { zr = O::sqr(x); zi = O::sqr(y); }
+    else { zr = O::mul(x, x); zi = O::mul(y, y); }
+    IterT iter = 0;
+    for (;;) {
+        bool in;
+        if constexpr (sizeof(F) == 4) in = O::le(O::add(zr, zi), O::make(4.0f, 0, 0, 0));
+        else in = O::le(O::add(zr, zi), 4.0);
+        if (!(in && iter < n_iterations)) break;
+        y = O::mul(x, y);
+        if constexpr (sizeof(F) == 4) y = O::mul_pwr2(y, 2.0f);
+        else y = O::mul(y, 2.0);
+        y = O::add(y, y0);
+        x = O::add(O::sub(zr, zi), x0);
+        if constexpr (sizeof(F) == 4) { zr = O::sqr(x); zi = O::sqr(y); }
+        else { zr = O::mul(x, x); zi = O::mul(y, y); }
+        iter++;
+    }
+    return iter;
+}
 
 } // namespace fs

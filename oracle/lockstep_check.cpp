@@ -19,6 +19,7 @@
 #include "../fractalshark_b200/csrc/fs_la_fast.cuh"
 #include "../fractalshark_b200/csrc/fs_la_step2.cuh"
 #include "../fractalshark_b200/csrc/fs_num.cuh"
+#include "../fractalshark_b200/csrc/fs_qd.cuh"
 
 namespace {
 
@@ -556,6 +557,42 @@ int lockstep_numeric_op(uint32_t op, const void *a_, const void *b_, void *out_,
         }
     }
     return 0;
+}
+
+// The host build of the Quad<F> operations (fs_qd.cuh quad_selftest_op): the CPU pre-image of fs_selftest_numeric_op
+// 60-67 (Quad<double>, 32-byte elements) and 70-77 (Quad<float>, 16-byte elements).  -1: not a Quad op.
+int lockstep_quad_op(uint32_t op, const void *a_, const void *b_, void *out_, uint64_t n) {
+    if (op >= 60 && op <= 67) {
+        const fs::Quad<double> *a = (const fs::Quad<double> *)a_, *b = (const fs::Quad<double> *)b_;
+        for (uint64_t i = 0; i < n; i++) ((fs::Quad<double> *)out_)[i] = fs::quad_selftest_op<double>(op - 60, a[i], b[i]);
+        return 0;
+    }
+    if (op >= 70 && op <= 77) {
+        const fs::Quad<float> *a = (const fs::Quad<float> *)a_, *b = (const fs::Quad<float> *)b_;
+        for (uint64_t i = 0; i < n; i++) ((fs::Quad<float> *)out_)[i] = fs::quad_selftest_op<float>(op - 70, a[i], b[i]);
+        return 0;
+    }
+    return -1;
+}
+
+// The escape-time loop of Gpu4x32 (limb_bytes 4) / Gpu4x64 (limb_bytes 8) -- fs_qd.cuh quad_escape_count, the code the
+// kernels run -- for `n` pixels given by their kernel coordinates (X[i], Y[i]) (Y already flipped).  out[i] = count.
+// Returns 0, or -1 for an unknown limb size.
+int lockstep_quad_pixels(int limb_bytes, int iter_bytes, const void *cx, const void *cy, const void *dx, const void *dy,
+                         uint64_t n_iterations, const int32_t *X, const int32_t *Y, uint64_t n, uint64_t *out, int threads) {
+    auto run = [&](auto limb, auto it) {
+        using F = decltype(limb);
+        using IterT = decltype(it);
+        fs::Quad<F> c[4];
+        memcpy(&c[0], cx, sizeof(c[0])); memcpy(&c[1], cy, sizeof(c[0]));
+        memcpy(&c[2], dx, sizeof(c[0])); memcpy(&c[3], dy, sizeof(c[0]));
+        parallel_rows(0, (int)n, threads, [&](int i) {
+            out[i] = (uint64_t)fs::quad_escape_count<F, IterT>(c[0], c[1], c[2], c[3], X[i], Y[i], (IterT)n_iterations);
+        });
+    };
+    if (limb_bytes == 4) { if (iter_bytes == 8) run(0.0f, uint64_t{}); else run(0.0f, uint32_t{}); return 0; }
+    if (limb_bytes == 8) { if (iter_bytes == 8) run(0.0, uint64_t{}); else run(0.0, uint32_t{}); return 0; }
+    return -1;
 }
 
 } // extern "C"

@@ -164,3 +164,108 @@ def mismatches(got, want):
             got[f][both] = 0
             want[f][both] = 0
     return np.flatnonzero((got.view(np.uint8).reshape(n, -1) != want.view(np.uint8).reshape(n, -1)).any(axis=1))
+
+
+# ---- Quad<F> (fs_qd.cuh) --------------------------------------------------------------------------------------------
+# Listed apart from OPS: these operations have no bit-exact restatement in the oracle by design (the port splits products
+# with an FMA where the reference leaves a Dekker split to the compiler).  They are checked against exact arithmetic
+# within the bounds of tests/exact_escape.py, and the device against the host build of fs_qd.cuh bit for bit.
+QUAD_OPS = [
+    (60, "Quad<double> add"), (61, "Quad<double> sub"), (62, "Quad<double> mul(q, q)"), (63, "Quad<double> mul(q, scalar)"),
+    (64, "Quad<double> sqr"), (65, "Quad<double> mul_pwr2"), (66, "Quad<double> le(q, q)"), (67, "Quad<double> le(q, scalar)"),
+    (70, "Quad<float> add"), (71, "Quad<float> sub"), (72, "Quad<float> mul(q, q)"), (73, "Quad<float> mul(q, scalar)"),
+    (74, "Quad<float> sqr"), (75, "Quad<float> mul_pwr2"), (76, "Quad<float> le(q, q)"), (77, "Quad<float> le(q, scalar)"),
+]
+_Q64 = np.dtype([("x", "<f8"), ("y", "<f8"), ("z", "<f8"), ("w", "<f8")])
+_Q32 = np.dtype([("x", "<f4"), ("y", "<f4"), ("z", "<f4"), ("w", "<f4")])
+
+
+def quad_dtype(op):
+    return _Q64 if op < 70 else _Q32
+
+
+def _expansion(value, ft):
+    """Greedy round-to-nearest four-limb expansion of the Fraction `value` (normalised: each limb rounds what is left)."""
+    from fractions import Fraction
+    limbs, rest = [], value
+    for _ in range(4):
+        v = ft(float(rest)) if rest != 0 else ft(0.0)
+        limbs.append(v)
+        rest -= Fraction(float(v))
+    return limbs
+
+
+def quad_operands(op, n):
+    """Operand pairs for the Quad<F> operation `op`, aimed at the case distinctions of fs_qd.cuh: zero limbs (the zero
+    shortcuts of two_sum / quick_two_sum / renorm in the double flavour), cancellation a ~ -b to every limb depth,
+    overlapping and widely spaced limbs, sums and squares around the bailout |z|^2 ~ 4, tiny magnitudes where the low
+    limbs of Quad<float> are subnormal, signed zeros, and for le equal heads (and equal second / third limbs).
+    The scalar operand of ops 3, 5, 7 is b.x."""
+    from fractions import Fraction
+    rng = np.random.default_rng(2000 + op)
+    k = op % 10
+    dt = quad_dtype(op)
+    ft = dt["x"].type
+    p = 53 if op < 70 else 24
+    a, b = np.zeros(n, dt), np.zeros(n, dt)
+
+    def rand_value(lo, hi):
+        # a value with far more bits than four limbs hold, magnitude 2^[lo, hi)
+        m = Fraction(int(rng.integers(1 << 62, 1 << 63)), 1 << 62) + Fraction(int(rng.integers(0, 1 << 62)), 1 << 124)
+        m += Fraction(int(rng.integers(0, 1 << 62)), 1 << 186) + Fraction(int(rng.integers(0, 1 << 62)), 1 << 248)
+        m *= Fraction(2) ** int(rng.integers(lo, hi))
+        return m if rng.integers(0, 2) else -m
+
+    tiny_lo = -140 if op >= 70 else -300
+    for i in range(n):
+        kind = int(rng.integers(0, 10))
+        if kind == 6 and op >= 70:
+            lo, hi = tiny_lo, -40                         # Quad<float>: third / fourth limbs subnormal
+        elif kind == 5:
+            lo, hi = 0, 2                                 # around the bailout: |a|, |b| in [1, 4)
+        else:
+            lo, hi = -12, 4
+        va, vb = rand_value(lo, hi), rand_value(lo, hi)
+        la, lb = _expansion(va, ft), _expansion(vb, ft)
+        if kind == 0:                                     # zero limbs
+            for L in (la, lb):
+                for j in range(1, 4):
+                    if rng.integers(0, 2):
+                        L[j] = ft(0.0)
+            if rng.integers(0, 4) == 0:
+                la = [ft(0.0)] * 4
+        elif kind == 1 and k in (0, 1):                   # cancellation a ~ -b (add) / a ~ b (sub) down to limb `d`
+            d = int(rng.integers(1, 5))
+            s = -1 if k == 0 else 1
+            lb = [ft(s * v) for v in la[:d]] + lb[d:] if d < 4 else [ft(s * v) for v in la]
+            if d < 4:
+                rest = _expansion(rand_value(lo - p * d, hi - p * d), ft)
+                lb = lb[:d] + rest[:4 - d]
+        elif kind == 2:                                   # overlapping limbs: y within 2^-8 of x's magnitude
+            la[1] = ft(float(la[0]) * float(rng.uniform(-1, 1)) * 2.0 ** -int(rng.integers(1, 9)))
+        elif kind == 3:                                   # widely spaced limbs
+            for j in range(1, 4):
+                la[j] = ft(float(la[j]) * 2.0 ** -int(rng.integers(0, 2 * p)))
+        elif kind == 4:                                   # signed zeros: trailing limbs (or all four) +-0
+            for L in (la, lb):
+                d = int(rng.integers(0, 4))
+                for j in range(d, 4):
+                    L[j] = ft(-0.0) if rng.integers(0, 2) else ft(0.0)
+        if k in (6, 7):                                   # the comparison is specified on normalised expansions
+            la = _expansion(sum((Fraction(float(v)) for v in la), Fraction(0)), ft)
+            lb = _expansion(sum((Fraction(float(v)) for v in lb), Fraction(0)), ft)
+            if rng.integers(0, 2):                        # equal heads, and equal second / third / fourth limbs
+                d = int(rng.integers(1, 5))
+                vb = sum((Fraction(float(v)) for v in la[:d]), Fraction(0))
+                if d < 4 and la[d - 1] != 0 and rng.integers(0, 4):
+                    vb += rand_value(-2 * p, -p - 1) * Fraction(abs(float(la[d - 1])))
+                lb = _expansion(vb, ft)
+            if kind == 4:
+                la = [ft(-0.0) if v == 0 else v for v in la]
+        a[i] = tuple(la)
+        b[i] = tuple(lb)
+    if k == 5:                                            # mul_pwr2: the kernel doubles; halving may round subnormals
+        b["x"] = rng.choice(np.array([2.0, 2.0, 2.0, -2.0, 4.0, 0.5]), n).astype(ft)
+    if k == 7:
+        b["x"] = np.where(rng.integers(0, 2, n) == 0, a["x"], b["x"])   # le(q, scalar) with a.x == b
+    return a, b

@@ -287,3 +287,38 @@ def lockstep_numeric_op(op: int, a: np.ndarray, b: np.ndarray) -> np.ndarray:
     rc = fn(op, a.ctypes.data, b.ctypes.data, out.ctypes.data, a.shape[0])
     assert rc == 0, rc
     return out
+
+
+def lockstep_quad_op(op: int, a: np.ndarray, b: np.ndarray) -> np.ndarray:
+    """The host build of the Quad<F> operations (fs_qd.cuh quad_selftest_op, ops 60-67 / 70-77) on operand arrays."""
+    global _lock
+    if _lock is None:
+        _lock = C.CDLL(LOCKSTEP_LIB)
+    fn = _lock.lockstep_quad_op
+    fn.restype = C.c_int
+    fn.argtypes = [C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
+    a = np.ascontiguousarray(a)
+    b = np.ascontiguousarray(b)
+    out = np.zeros_like(a)
+    rc = fn(op, a.ctypes.data, b.ctypes.data, out.ctypes.data, a.shape[0])
+    assert rc == 0, rc
+    return out
+
+
+def quad_escape_counts(limb_bytes, coords, n_iter, X, Y, iter_bytes=4, threads=1):
+    """The escape-time loop of Gpu4x32 (limb_bytes 4) / Gpu4x64 (8) -- fs_qd.cuh quad_escape_count, host build -- for the
+    kernel pixels (X[i], Y[i]) (Y: the kernel's own, flipped row).  Returns the counts as uint64."""
+    global _lock
+    if _lock is None:
+        _lock = C.CDLL(LOCKSTEP_LIB)
+    fn = _lock.lockstep_quad_pixels
+    fn.restype = C.c_int
+    V = C.c_void_p
+    fn.argtypes = [C.c_int, C.c_int, V, V, V, V, C.c_uint64, V, V, C.c_uint64, V, C.c_int]
+    X = np.ascontiguousarray(X, dtype=np.int32)
+    Y = np.ascontiguousarray(Y, dtype=np.int32)
+    out = np.zeros(X.shape[0], np.uint64)
+    rc = fn(limb_bytes, iter_bytes, _buf(coords["cx"]), _buf(coords["cy"]), _buf(coords["dx"]), _buf(coords["dy"]), n_iter,
+            X.ctypes.data, Y.ctypes.data, X.shape[0], out.ctypes.data, threads)
+    assert rc == 0, rc
+    return out

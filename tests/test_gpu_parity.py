@@ -111,19 +111,6 @@ def test_full_size_vs_reference_cuda_kernels(case):
     assert (red["Min"], red["Max"], red["Sum"]) == (ref_red["Min"], ref_red["Max"], ref_red["Sum"]) or min_exact < 1.0
 
 
-def test_four_limb_kernels_resolve_what_double_double_resolves():
-    """Property for Gpu4x64 where the reference's own 4x64 kernel cannot serve as the checker (on windows of
-    width 1e-24 its frame is one constant -- it resolves less than its 2x64 kernel): the four-double kernel
-    must agree with the double-double kernel (itself bit-exact against the reference) on a window both resolve."""
-    w, h, n = 480, 270, 20000
-    _, c2, _, _, _ = cases.make_inputs(102, w, h, A.Gpu2x64, n, 4)
-    _, c4, _, _, _ = cases.make_inputs(102, w, h, A.Gpu4x64, n, 4)
-    i2, _, _ = cases.render(GPURenderer, w, h, A.Gpu2x64, c2, None, None, n, 4)
-    i4, _, _ = cases.render(GPURenderer, w, h, A.Gpu4x64, c4, None, None, n, 4)
-    assert float((i2[:h, :w] == i4[:h, :w]).mean()) >= 0.999
-    assert int(i4[:h, :w].max()) > int(i4[:h, :w].min())
-
-
 def test_full_size_properties_without_reference():
     """Size-independent properties at 3840x2160: idempotence, sharded == unsharded, checksum of checksums,
     u32 == u64, sampled rows == oracle."""
