@@ -987,6 +987,19 @@ __global__ void numeric_op_kernel(uint32_t op, const void *a_, const void *b_, v
         static_cast<Wire *>(out_)[i] = Wire{r.m, r.e, 0};
         break;
     }
+    case 80: case 81: case 82: case 83: case 84: case 85: { // perturbation policies, 128-byte records (fs_num.cuh)
+        const unsigned char *in = static_cast<const unsigned char *>(a_) + (size_t)kPerturbRecordBytes * i;
+        unsigned char *o = static_cast<unsigned char *>(out_) + (size_t)kPerturbRecordBytes * i;
+        switch (op) {
+        case 80: perturb_selftest<NumPlain<float>>(in, o); break;
+        case 81: perturb_selftest<NumPlain<double>>(in, o); break;
+        case 82: perturb_selftest<NumHdr<float>>(in, o); break;
+        case 83: perturb_selftest<NumHdr<double>>(in, o); break;
+        case 84: perturb_selftest<Num2x32>(in, o); break;
+        default: perturb_selftest<NumHdr2x32>(in, o); break;
+        }
+        break;
+    }
     case 30: static_cast<dd64 *>(out_)[i] = dd_add(qa[i], qb[i]); break;
     case 31: static_cast<dd64 *>(out_)[i] = dd_sub(qa[i], qb[i]); break;
     case 32: static_cast<dd64 *>(out_)[i] = dd_mul(qa[i], qb[i]); break;
@@ -1010,6 +1023,7 @@ uint32_t numeric_op_elem_bytes(uint32_t op) {
     if (op >= 50 && op <= 56) return 16;
     if (op >= 60 && op <= 67) return 32;
     if (op >= 70 && op <= 77) return 16;
+    if (op >= 80 && op <= 85) return kPerturbRecordBytes;
     return 0;
 }
 } // namespace

@@ -123,4 +123,28 @@ template <class M> struct NumHdr {
     FS_HD static Real delta_y(Real dy, int Y, Real centerY) { return sub(mul(neg(dy), from_int(Y)), centerY); }
 };
 
+// Per-step self-test of a perturbation policy (fs_selftest_numeric_op 80-85, host: lockstep_numeric_op 80-83): one
+// record of 8 cells of 16 bytes, each cell one Real in its in-memory layout.  In: dx, dy, zx, zy, dcx, dcy,
+// {int32 X, int32 Y}.  Out: perturb(dx, dy, zx, zy, dcx, dcy) in cells 0-1, norm2(dx, dy) in 2,
+// delta_x(zx, X, dcx) in 3, delta_y(zy, Y, dcy) in 4, add(zx, dx) in 5.  tests/test_exact_perturb.py holds each
+// result to the bound of tests/exact_perturb.py.  (Num2x32 / NumHdr2x32 are device-only.)
+constexpr int kPerturbRecordBytes = 128;
+template <class Num> FS_HD void perturb_selftest(const unsigned char *in, unsigned char *out) {
+    using Real = typename Num::Real;
+    static_assert(sizeof(Real) <= 16, "one cell per number");
+    Real v[6], r[6];
+    for (int k = 0; k < 6; k++) memcpy(&v[k], in + 16 * k, sizeof(Real));
+    int32_t xy[2];
+    memcpy(xy, in + 96, sizeof(xy));
+    r[0] = v[0];
+    r[1] = v[1];
+    Num::perturb(r[0], r[1], v[2], v[3], v[4], v[5]);
+    r[2] = Num::norm2(v[0], v[1]);
+    r[3] = Num::delta_x(v[2], xy[0], v[4]);
+    r[4] = Num::delta_y(v[3], xy[1], v[5]);
+    r[5] = add(v[2], v[0]);
+    for (int k = 0; k < kPerturbRecordBytes; k++) out[k] = 0;
+    for (int k = 0; k < 6; k++) memcpy(out + 16 * k, &r[k], sizeof(Real));
+}
+
 } // namespace fs

@@ -547,6 +547,15 @@ int lockstep_numeric_op(uint32_t op, const void *a_, const void *b_, void *out_,
             ((Wire *)out_)[i] = Wire{q.m, q.e, 0};
             break;
         }
+        case 80: case 81: case 82: case 83: { // perturbation policies (fs_num.cuh perturb_selftest), 128-byte records
+            const unsigned char *in = (const unsigned char *)a_ + (size_t)fs::kPerturbRecordBytes * i;
+            unsigned char *o = (unsigned char *)out_ + (size_t)fs::kPerturbRecordBytes * i;
+            if (op == 80) fs::perturb_selftest<fs::NumPlain<float>>(in, o);
+            else if (op == 81) fs::perturb_selftest<fs::NumPlain<double>>(in, o);
+            else if (op == 82) fs::perturb_selftest<fs::NumHdr<float>>(in, o);
+            else fs::perturb_selftest<fs::NumHdr<double>>(in, o);
+            break;
+        }
         case 40: {
             fs::Hdr<float> dx = hf(fa[3 * i]), dy = hf(fa[3 * i + 1]);
             fs::NumHdr<float>::perturb(dx, dy, hf(fa[3 * i + 2]), hf(fb[3 * i]), hf(fb[3 * i + 1]), hf(fb[3 * i + 2]));

@@ -1,4 +1,4 @@
-"""Exact escape-time reference for the direct kernels (Gpu1x32, Gpu1x64, Gpu2x32, Gpu2x64, Gpu4x32, Gpu4x64).
+"""Exact escape-time reference for the direct kernels (Gpu1x32, Gpu1x64, Gpu2x32, Gpu2x64, Gpu4x32, Gpu4x64, GpuHDRx32).
 
 Pure Python, no native code.  For a pixel with c = (cx + X dx, cy + Y dy) -- the coordinate PODs decoded exactly as the
 sum of their limbs, Y the kernel's own (flipped) row -- z <- z^2 + c is iterated on integers in fixed point with
@@ -35,6 +35,8 @@ class ArithModel:
                 |computed - exact| <= eps * (sum of the operands' magnitudes) for add/sub, eps * |a||b| for products,
                 eps * |a|^2 for squares, eps * |a||s| for a number times a limb, each plus floor_op
     floor_op    absolute error floor of one operation (underflow into the subnormal range of the lowest limbs)
+    hdr         HDRFloat<CudaDblflt> (GpuHDRx32): fed an HDRFloat<double> POD {f64 m, int32 exp, pad}, which the C-ABI
+                splits into head = (float)m, tail = (float)(m - head), renormalised exactly (fs_capi.cu hdr2x32_from_hdr64)
     """
     name: str
     limb_bits: int
@@ -45,6 +47,7 @@ class ArithModel:
     eps_sqr: float
     eps_scal: float
     floor_op: float
+    hdr: bool = False
 
     @property
     def u(self) -> float:
@@ -82,7 +85,14 @@ DD64 = ArithModel("dd64", 53, 2, _F64_SUB, 4 * 2.0 ** -106, 8 * 2.0 ** -106, 8 *
 QF32 = ArithModel("qf32", 24, 4, _F32_SUB, 16 * 2.0 ** -96, 48 * 2.0 ** -96, 48 * 2.0 ** -96, 16 * 2.0 ** -96, 16 * _F32_SUB)
 QD64 = ArithModel("qd64", 53, 4, _F64_SUB, 16 * 2.0 ** -212, 48 * 2.0 ** -212, 48 * 2.0 ** -212, 16 * 2.0 ** -212,
                   16 * _F64_SUB)
-MODELS = {m.name: m for m in (F32, F64, DF32, DD64, QF32, QD64)}
+# HDR over 2x32 (GpuHDRx32): the mantissa operations are dblflt's (the DF32 bounds, checked through
+# fs_selftest_numeric_op 85 as well); the exponent removes underflow.  What is left as an absolute floor: operands
+# dropped at exponent gaps >= 120 (below 2^-115 for the values |v| < 32 of an iteration that has not escaped) and
+# Reduce's rebasing of a zero tail, which leaves it as 2^(-k - 127) for a head of exponent -k < 0 (fs_df32.cuh
+# reduce, the reference's): a relative error below 2^-125 per Reduce.
+HDF32 = ArithModel("hdf32", 24, 2, 0.0, 4 * 2.0 ** -48, 8 * 2.0 ** -48, 8 * 2.0 ** -48, 8 * 2.0 ** -48, 2.0 ** -100,
+                   hdr=True)
+MODELS = {m.name: m for m in (F32, F64, DF32, DD64, QF32, QD64, HDF32)}
 
 
 @dataclass(frozen=True)
@@ -91,7 +101,7 @@ class Kernel:
 
     strict      bailout `value < 4` (True) or `value <= 4` (False)
     cap_minus   the limit is n_iterations - (P - 1) (the 1x kernels) instead of n_iterations
-    step        which step the kernel executes ('1x', '2x32', '2x64', '4x32', '4x64')
+    step        which step the kernel executes ('1x', '2x32', '2x64', '4x32', '4x64', 'hdr2x32')
     """
     name: str
     model: ArithModel
@@ -108,25 +118,49 @@ KERNELS = {
     "Gpu2x64": Kernel("Gpu2x64", DD64, True, False, "2x64", (1,)),           # __dadd_rn(zr.head, zi.head) < 4
     "Gpu4x32": Kernel("Gpu4x32", QF32, False, False, "4x32", (1,)),          # le(add(zr, zi), 4)
     "Gpu4x64": Kernel("Gpu4x64", QD64, False, False, "4x64", (1,)),
+    "GpuHDRx32": Kernel("GpuHDRx32", HDF32, True, False, "hdr2x32", (1, 4, 8, 16)),  # cmp_pr(reduced |z|^2, 4) < 0
 }
 
 
 # ---- coordinate PODs ----------------------------------------------------------------------------------------------
+def _f32(v: float) -> float:
+    return struct.unpack("<f", struct.pack("<f", v))[0]
+
+
 def pod_limbs(raw: bytes, model: ArithModel) -> list:
-    """The limbs of one coordinate POD (little-endian binary32 / binary64 limbs, most significant first)."""
+    """The limbs of one coordinate POD (little-endian binary32 / binary64 limbs, most significant first); HDR: the
+    head and tail the kernel holds, without the exponent."""
+    if model.hdr:
+        m = struct.unpack("<d", raw[:8])[0]
+        a = _f32(m)
+        return [a, _f32(m - a)]
     fmt = "<%d%s" % (model.limbs, "f" if model.limb_bits == 24 else "d")
     return list(struct.unpack(fmt, raw))
 
 
 def pod_value(raw: bytes, model: ArithModel) -> Fraction:
-    """The exact value of a coordinate POD: the sum of its limbs as dyadic rationals."""
-    return sum((Fraction(v) for v in pod_limbs(raw, model)), Fraction(0))
+    """The exact value of a coordinate POD as the kernel holds it: the sum of its limbs as dyadic rationals (HDR: times
+    2^exp)."""
+    v = sum((Fraction(v) for v in pod_limbs(raw, model)), Fraction(0))
+    if model.hdr:
+        v *= Fraction(2) ** struct.unpack("<i", raw[8:12])[0]
+    return v
 
 
 def pack_pod(value, model: ArithModel) -> bytes:
-    """A POD whose limbs are the greedy round-to-nearest expansion of `value` (exact for dyadic values that fit)."""
+    """A POD whose limbs are the greedy round-to-nearest expansion of `value` (exact for dyadic values that fit); HDR:
+    of the mantissa in [1, 2), or the zero at MIN_BIG."""
     rest, limbs = Fraction(value), []
     fmt = "f" if model.limb_bits == 24 else "d"
+    if model.hdr:
+        if rest == 0:
+            return struct.pack("<di4x", 0.0, -(2 ** 31) >> 3)
+        e = 0
+        while abs(rest) >= 2:
+            rest, e = rest / 2, e + 1
+        while abs(rest) < 1:
+            rest, e = rest * 2, e - 1
+        return struct.pack("<di4x", float(rest), e)
     for _ in range(model.limbs):
         v = float(rest)
         if fmt == "f":
@@ -172,14 +206,17 @@ def _step_errors(k: Kernel, ax: float, ay: float, ax0: float, ay0: float):
         # fma(x, x, fl(y*y)): two roundings to nearest
         et = 2 * u * (1 + 2 * u) * (x2 + y2) + 2 * fl
         return ex, ey, et
-    if k.step in ("2x32", "2x64"):
+    if k.step in ("2x32", "2x64", "hdr2x32"):
         eA, eM, eS = m.eps_add, m.eps_mul, m.eps_sqr
-        eZ = eS if k.step == "2x32" else eM        # zr = df_sqr(x) / dd_mul(x, x)
+        eZ = eS if k.step == "2x32" else eM        # zr = df_sqr(x) / dd_mul(x, x) / mul(x, x)
         mag = (1 + 4 * u)                           # |head| + |tail| vs |value|
         # x' = add(sub(zr, zi), x0): zr, zi carry their own rounding into the next step
         ex = (eZ * (x2 + y2) + eA * 2 * (x2 + y2) * (1 + eZ) + eA * ax0) * mag * mag + 5 * fl
         # y' = add(2 * mul(x, y), y0)  (the doubling is exact)
         ey = (2 * eM * xy + eA * (2 * xy * (1 + eM) + ay0)) * mag * mag + 3 * fl
+        if k.step == "hdr2x32":
+            # zs = reduced(add(zr, zi)), compared in full (cmp_pr)
+            return ex, ey, (eZ * (x2 + y2) + eA * (x2 + y2) * (1 + eZ)) * mag * mag + 3 * fl
         # zr.head + zi.head, rounded: |zr - zr.head| <= u |zr.head|, one more rounding of the sum
         et = (3 * u * (x2 + y2)) * mag * mag + 3 * fl
         return ex, ey, et
@@ -243,6 +280,8 @@ def escape_count(k: Kernel, cx: Fraction, cy: Fraction, dx: Fraction, dy: Fracti
         if exact:
             v = x * x + y * y                     # exact value of the test at 2P fraction bits
             F4 = FOUR << P
+            if v == F4 and m.hdr:
+                return it, False                  # a tie: decided by the last-bit residue Reduce leaves (HDF32)
             go_on = v < F4 if k.strict else v <= F4
             if not go_on:
                 return it, True
@@ -309,14 +348,20 @@ def escape_counts(kernel: str, coords, pixels, n_iterations: int, precision: int
                   processes: int | None = None):
     """escape_count over a list of kernel pixels (X, Y), spread over processes of a `spawn` context (safe after CUDA
     initialisation).  coords = (cx, cy, dx, dy) as Fractions.  Returns [(count, certified)]."""
+    return map_pixels(_work, lambda part: (kernel, tuple(coords), part, n_iterations, precision, model), pixels,
+                      processes)
+
+
+def map_pixels(work, job, pixels, processes: int | None = None):
+    """[work(job(part)) for the parts of `pixels`], flattened, on processes of a `spawn` context (safe after CUDA
+    initialisation).  `work` must be a module-level function; job(part) builds its picklable argument."""
     pixels = list(pixels)
     processes = processes or mp.cpu_count()
     chunk = max(1, len(pixels) // (processes * 8))
-    jobs = [(kernel, tuple(coords), pixels[i:i + chunk], n_iterations, precision, model)
-            for i in range(0, len(pixels), chunk)]
+    jobs = [job(pixels[i:i + chunk]) for i in range(0, len(pixels), chunk)]
     if processes == 1 or len(jobs) == 1:
-        res = [_work(j) for j in jobs]
+        res = [work(j) for j in jobs]
     else:
         with mp.get_context("spawn").Pool(processes) as pool:
-            res = pool.map(_work, jobs)
+            res = pool.map(work, jobs)
     return [r for part in res for r in part]

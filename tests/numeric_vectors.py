@@ -1,6 +1,10 @@
 """Operand vectors for the per-operation checks of the device numeric types (SURVEY section 8 row a8): HDRFloat<float>,
 HDRFloatComplex<float>, dblflt, dbldbl.  Used by the GPU suite (fs_selftest_numeric_op vs the oracle) and by the CPU suite
 (the host build of the same product headers vs the oracle)."""
+import math
+import struct
+from fractions import Fraction
+
 import numpy as np
 
 _HF = np.dtype([("m", "<f4"), ("e", "<i4")])
@@ -186,7 +190,6 @@ def quad_dtype(op):
 
 def _expansion(value, ft):
     """Greedy round-to-nearest four-limb expansion of the Fraction `value` (normalised: each limb rounds what is left)."""
-    from fractions import Fraction
     limbs, rest = [], value
     for _ in range(4):
         v = ft(float(rest)) if rest != 0 else ft(0.0)
@@ -201,7 +204,6 @@ def quad_operands(op, n):
     overlapping and widely spaced limbs, sums and squares around the bailout |z|^2 ~ 4, tiny magnitudes where the low
     limbs of Quad<float> are subnormal, signed zeros, and for le equal heads (and equal second / third limbs).
     The scalar operand of ops 3, 5, 7 is b.x."""
-    from fractions import Fraction
     rng = np.random.default_rng(2000 + op)
     k = op % 10
     dt = quad_dtype(op)
@@ -269,3 +271,123 @@ def quad_operands(op, n):
     if k == 7:
         b["x"] = np.where(rng.integers(0, 2, n) == 0, a["x"], b["x"])   # le(q, scalar) with a.x == b
     return a, b
+
+
+# ---- perturbation-step records (fs_num.cuh perturb_selftest, ops 80-85) ---------------------------------------------
+PERTURB_OPS = {"f32": 80, "f64": 81, "hdr32": 82, "hdr64": 83, "2x32": 84, "hdr2x32": 85}
+_CELL = {"f32": "<f", "f64": "<d", "2x32": "<ff", "hdr32": "<fi", "hdr64": "<di4x", "hdr2x32": "<ffi"}
+_GAPS = [0, 1, -1, 119, 120, 121, 126, 127, 128]
+
+
+def _f32(v):
+    return struct.unpack("<f", struct.pack("<f", v))[0]
+
+
+def _number(rng, tname, scale, zero_e=None):
+    """(cell bytes, exact value) of one number of about 2^scale; with zero_e an exact zero instead (HDR: at exponent
+    zero_e, or at the canonical MIN_BIG for zero_e == "canon")."""
+    hdr = tname.startswith("hdr")
+    sign = -1.0 if rng.integers(0, 2) else 1.0
+    if zero_e is not None:
+        if hdr:
+            e = _MIN_BIG if zero_e == "canon" else int(zero_e)
+            vals = {"hdr32": (0.0, e), "hdr64": (0.0, e), "hdr2x32": (0.0, 0.0, e)}[tname]
+        else:
+            vals = {"f32": (sign * 0.0,), "f64": (sign * 0.0,), "2x32": (0.0, 0.0)}[tname]
+        return struct.pack(_CELL[tname], *vals).ljust(16, b"\0"), Fraction(0)
+    if hdr:
+        # reduced mantissa in [1, 2), or an unreduced one in [2^-24, 8) as the kernels hold between Reduce calls
+        m = float(rng.uniform(1.0, 2.0)) if rng.integers(0, 3) else float(rng.uniform(1.0, 2.0)) * 2.0 ** int(rng.integers(-24, 3))
+        m *= sign
+        if tname == "hdr32":
+            m = _f32(m)
+            vals, v = (m, scale), Fraction(m) * Fraction(2) ** scale
+        elif tname == "hdr64":
+            vals, v = (m, scale), Fraction(m) * Fraction(2) ** scale
+        else:
+            h = _f32(m)
+            t = _f32(h * float(rng.uniform(-1, 1)) * 2.0 ** -25)
+            vals, v = (h, t, scale), (Fraction(h) + Fraction(t)) * Fraction(2) ** scale
+        return struct.pack(_CELL[tname], *vals).ljust(16, b"\0"), v
+    x = sign * float(rng.uniform(1.0, 2.0)) * 2.0 ** scale
+    if tname == "f32":
+        x = _f32(x)
+        return struct.pack("<f", x).ljust(16, b"\0"), Fraction(x)
+    if tname == "f64":
+        return struct.pack("<d", x).ljust(16, b"\0"), Fraction(x)
+    h = _f32(x)
+    t = _f32(h * float(rng.uniform(-1, 1)) * 2.0 ** -25)
+    return struct.pack("<ff", h, t).ljust(16, b"\0"), Fraction(h) + Fraction(t)
+
+
+def perturb_records(tname, n, seed=80):
+    """n records of perturb_selftest for the type and their exact operand values [(dx, dy, zx, zy, cx, cy, X, Y)],
+    aimed at the case distinctions of the step: exponent gaps 0, +-1, 119-121, 126-128 between the orbit, the delta and
+    dc; exact zeros (HDR: canonical, and at exponents up to the largest operand's, where a cancellation leaves them);
+    unreduced HDR mantissas;
+    subnormal results for the plain types; cancellation 2Z ~ -d and dc ~ -d (2Z + d)."""
+    rng = np.random.default_rng(seed)
+    hdr = tname.startswith("hdr")
+    lo = {"f32": -140, "2x32": -100, "f64": -1000}.get(tname, -100000)
+    rec = np.zeros((n, 128), np.uint8)
+    vals = []
+    for i in range(n):
+        sz = int(rng.integers(-40, 2)) if rng.integers(0, 4) == 0 else int(rng.integers(-2, 2))
+        g = _GAPS[int(rng.integers(0, len(_GAPS)))] if rng.integers(0, 2) else int(rng.integers(2, 60))
+        sd = max(sz - g, lo)
+        g2 = _GAPS[int(rng.integers(0, len(_GAPS)))] if rng.integers(0, 3) == 0 else int(rng.integers(-3, 4))
+        sc = max(min(sd + g2, 1), lo)
+        cells, v = [], []
+        for k, s in enumerate((sd, sd + int(rng.integers(-3, 4)), sz, sz + int(rng.integers(-3, 1)), sc, sc)):
+            s = max(s, lo)
+            z = None
+            if rng.integers(0, 12) == 0:
+                z = "canon" if (not hdr or rng.integers(0, 2)) else max(sz, sd, sc) + int(rng.integers(-200, 1))
+            c, x = _number(rng, tname, s, z)
+            cells.append(c)
+            v.append(x)
+        kind = int(rng.integers(0, 7))
+        if kind == 0 and v[2] != 0:     # 2 Zx ~ -dx: the delta cancels the orbit
+            tgt = -2 * v[2] * (1 + Fraction(int(rng.integers(-4, 5)), 1 << 30))
+            cells[0], v[0] = _pack_value(tname, tgt)
+        elif kind == 1:                 # dc ~ -d (2Z + d): the step cancels to nearly nothing
+            dx, dy, zx, zy = v[0], v[1], v[2], v[3]
+            ex = dx * (2 * zx + dx) - dy * (2 * zy + dy)
+            ey = dx * (2 * zy + dy) + dy * (2 * zx + dx)
+            if ex != 0:
+                cells[4], v[4] = _pack_value(tname, -ex)
+            if ey != 0:
+                cells[5], v[5] = _pack_value(tname, -ey)
+        X, Y = int(rng.integers(0, 5000)), int(rng.integers(0, 5000))
+        buf = b"".join(cells) + struct.pack("<ii", X, Y)
+        rec[i, :len(buf)] = np.frombuffer(buf, np.uint8)
+        vals.append((*v, X, Y))
+    return rec, vals
+
+
+def _pack_value(tname, q):
+    """(cell, exact value) of the type's nearest representation of the rational q (HDR: reduced mantissa)."""
+    if q == 0:
+        return _number(np.random.default_rng(0), tname, 0, "canon")
+    if tname in ("f32", "f64"):
+        x = _f32(float(q)) if tname == "f32" else float(q)
+        return struct.pack(_CELL[tname], x).ljust(16, b"\0"), Fraction(x)
+    if tname == "2x32":
+        h = _f32(float(q))
+        t = _f32(float(q - Fraction(h)))
+        return struct.pack("<ff", h, t).ljust(16, b"\0"), Fraction(h) + Fraction(t)
+    e = math.floor(math.log2(abs(q))) if abs(q) > 0 else 0
+    while abs(q) >= Fraction(2) ** (e + 1):
+        e += 1
+    while abs(q) < Fraction(2) ** e:
+        e -= 1
+    m = q / Fraction(2) ** e
+    if tname == "hdr32":
+        mm = _f32(float(m))
+        return struct.pack("<fi", mm, e).ljust(16, b"\0"), Fraction(mm) * Fraction(2) ** e
+    if tname == "hdr64":
+        mm = float(m)
+        return struct.pack("<di4x", mm, e).ljust(16, b"\0"), Fraction(mm) * Fraction(2) ** e
+    h = _f32(float(m))
+    t = _f32(float(m - Fraction(h)))
+    return struct.pack("<ffi", h, t, e).ljust(16, b"\0"), (Fraction(h) + Fraction(t)) * Fraction(2) ** e

@@ -21,9 +21,11 @@ from fractalshark_b200 import RenderAlgorithm as A
 from fractalshark_b200.views import PRESETS, VIEW1, ViewPreset
 
 ALGS = {"Gpu1x32": A.Gpu1x32, "Gpu1x64": A.Gpu1x64, "Gpu2x32": A.Gpu2x32, "Gpu2x64": A.Gpu2x64, "Gpu4x32": A.Gpu4x32,
-        "Gpu4x64": A.Gpu4x64}
+        "Gpu4x64": A.Gpu4x64, "GpuHDRx32": A.GpuHDRx32}
 TAGS = {"Gpu1x32": Numeric.F32, "Gpu1x64": Numeric.F64, "Gpu2x32": Numeric.X2_32, "Gpu2x64": Numeric.X2_64,
-        "Gpu4x32": Numeric.X4_32, "Gpu4x64": Numeric.X4_64}
+        "Gpu4x32": Numeric.X4_32, "Gpu4x64": Numeric.X4_64, "GpuHDRx32": Numeric.HDR64}
+# GpuHDRx32 (HDR over 2x32) has no CPU restatement: its arithmetic is device-only, so it is checked on the GPU
+CPU_KERNELS = [k for k in TAGS if k != "GpuHDRx32"]
 WORKERS = max(1, min(8, os.cpu_count() or 1))
 
 
@@ -48,22 +50,46 @@ def exact_view_coords(p: ViewPreset, w: int, h: int):
     return mnx, mny, (mxx - mnx) / w, (mxy - mny) / h
 
 
-@pytest.mark.parametrize("kernel", list(TAGS))
+# The perturbation kernels' PODs (fs_host.cpp fsh_view_coords): numeric tag, exact_perturb type, relative precision
+# (F32 / HDR32 round the mpf through binary64 to binary32: < 2^-23; F64 / HDR64: < 2^-52; X2_32 splits the binary64
+# value into head + rounded tail: < 2^-47; HDR2X32 splits the truncated 53-bit mpf mantissa into head and
+# (float)(m - head) without renormalising or reducing: the tail's rounding, 2^-24 of |m - head| <= 2^-24 |m|, and the
+# truncation, < 2^-47 of the value in all), subnormal floor.
+PO_TAGS = {"PO-F32": (Numeric.F32, "f32", 23, 2.0 ** -149), "PO-F64": (Numeric.F64, "f64", 52, 2.0 ** -1074),
+           "PO-X2_32": (Numeric.X2_32, "2x32", 47, 2 * 2.0 ** -149), "PO-HDR32": (Numeric.HDR32, "hdr32", 23, 0.0),
+           "PO-HDR64": (Numeric.HDR64, "hdr64", 52, 0.0), "PO-HDR2X32": (Numeric.HDR2X32, "hdr2x32", 47, 0.0)}
+
+
+@pytest.mark.parametrize("kernel", list(TAGS) + list(PO_TAGS))
 @pytest.mark.parametrize("view_id", [0, 1, 102, 103, 104])
 def test_view_coordinate_pods_hold_the_view_within_the_type_precision(built, kernel, view_id):
-    """View.coords: each POD (the numeric tag the direct kernel is fed: F32, F64, MattDblflt 0x102, X2_64, X4_32, X4_64)
-    equals the exact coordinate within the type's precision: L limbs of p bits, each limb the conversion of what the
+    """View.coords: each POD (the numeric tag the direct kernel is fed: F32, F64, MattDblflt 0x102, X2_64, X4_32, X4_64,
+    HDR64 split into 2x32 as GpuHDRx32 holds it) equals the exact coordinate within the type's precision: L limbs of p bits, each limb the
+    conversion of what the
     limbs before it left (truncated then rounded: < 2^-(p-1) relative per limb), plus one subnormal spacing per limb,
-    plus the error of the generator's own mpf arithmetic at View.precision_bits."""
+    plus the error of the generator's own mpf arithmetic at View.precision_bits.  The perturbation kernels' PODs
+    (PO-*: F32, F64, X2_32 as CudaDblflt, HDR32, HDR64, HDR2X32) are checked the same way, with center_x = C_x - minX
+    and center_y = C_y - maxY (C the view's centre): they are the exact model's starting radius (exact_perturb.py)."""
     from fractalshark_b200.host_inputs import View
     w, h = 320, 180
     p = PRESETS[view_id]
     view = View(p.min_x, p.min_y, p.max_x, p.max_y, w, h)
-    pods = view.coords(TAGS[kernel], direct=True)
-    m = E.KERNELS[kernel].model
     scale = max(abs(Fraction(s)) for s in (p.min_x, p.min_y, p.max_x, p.max_y))
     mpf_err = 16 * scale * Fraction(1, 2 ** view.precision_bits)
-    for name, want in zip(("cx", "cy", "dx", "dy"), exact_view_coords(p, w, h)):
+    cx, cy, dx, dy = exact_view_coords(p, w, h)
+    if kernel in PO_TAGS:
+        import exact_perturb as EP
+        tag, tname, bits, sub = PO_TAGS[kernel]
+        pods = view.coords(tag)
+        want = {"cx": cx, "cy": cy, "dx": dx, "dy": dy, "center_x": w * dx / 2, "center_y": -h * dy / 2}
+        for name, v in want.items():
+            got = EP.pod_value(tname, pods[name])
+            tol = abs(v) * Fraction(1, 2 ** bits) + Fraction(sub) + mpf_err
+            assert abs(got - v) <= tol, (name, float(got), float(v), float(abs(got - v) / tol))
+        return
+    pods = view.coords(TAGS[kernel], direct=True)
+    m = E.KERNELS[kernel].model
+    for name, want in zip(("cx", "cy", "dx", "dy"), (cx, cy, dx, dy)):
         got = E.pod_value(pods[name], m)
         tol = abs(want) * Fraction(1, 2 ** (m.limbs * (m.limb_bits - 1))) + m.limbs * Fraction(m.sub_min) + mpf_err
         assert abs(got - want) <= tol, (name, float(got), float(want), float(abs(got - want) / tol))
@@ -226,6 +252,7 @@ def edge_cases():
 
 
 EDGE_CASES = edge_cases()
+CPU_EDGE_CASES = [c for c in EDGE_CASES if c[0] in CPU_KERNELS]
 _EDGE_MODEL = {}
 
 
@@ -251,6 +278,9 @@ def _cap(kernel, P, n):
 # c -> expected count for P = 1: (1x and 2x kernels, 4x kernels); None = the cap
 EDGE_TABLE = {(-2, 0): (1, None), (0, 2): (1, 2), (2, 0): (1, 2), (1, 0): (2, 3), (-1, 1): (3, 3), (0, 1): (None, None),
               (-1, 0): (None, None), (0, 0): (None, None)}
+# the entries decided by a tie |z|^2 = 4: GpuHDRx32's Reduce leaves a last-bit residue in zero tails (exact_escape HDF32),
+# so the model does not certify ties for it
+EDGE_TIES = {(-2, 0), (0, 2), (2, 0), (1, 0)}
 
 
 def test_edge_table_is_what_the_exact_model_gives():
@@ -261,6 +291,8 @@ def test_edge_table_is_what_the_exact_model_gives():
         for n in (1, 2, 3, 37):
             cnt, cert = edge_model(kernel, 1, n)
             for (re, im), want in EDGE_TABLE.items():
+                if E.KERNELS[kernel].model.hdr and (re, im) in EDGE_TIES:
+                    continue
                 X, Y = (re + 2) * 4, (im + 2) * 4
                 w = want[1 if four else 0]
                 w = n if w is None else min(w, n)
@@ -285,7 +317,7 @@ def _cpu_edge(kernel, P, n, ib):
     return out[:EDGE_H, :EDGE_W]
 
 
-@pytest.mark.parametrize("kernel,P,n", EDGE_CASES, ids=["%s-p%d-n%d" % c for c in EDGE_CASES])
+@pytest.mark.parametrize("kernel,P,n", CPU_EDGE_CASES, ids=["%s-p%d-n%d" % c for c in CPU_EDGE_CASES])
 def test_edge_points_cpu(built, kernel, P, n):
     """The oracle's restatement (1x, 2x) / the host build of the four-limb loop on the exact 17 x 17 grid: every
     certified pixel equals the exact count, for 32- and 64-bit iteration types."""
@@ -338,6 +370,7 @@ WINDOWS = [
     ("4x64-v102", "Gpu4x64", PRESETS[102], 0.9, 12),
     ("4x64-v103", "Gpu4x64", PRESETS[103], 0.9, 12),
     ("4x32-v104", "Gpu4x32", PRESETS[104], 0.9, 12),
+    ("hdrx32-v1w3e-7", "GpuHDRx32", _around_view1(Fraction(3, 10 ** 7)), 0.9, 12),   # 2x32's 48 bits, as Gpu2x32
 ]
 WIN_IDS = [w[0] for w in WINDOWS]
 
@@ -347,6 +380,7 @@ def window_precisions(kernel):
 
 
 WIN_CASES = [(w[0], P) for w in WINDOWS for P in window_precisions(w[1])]
+CPU_WIN_CASES = [c for c in WIN_CASES if WINDOWS[WIN_IDS.index(c[0])][1] in CPU_KERNELS]
 
 
 def window_pixels():
@@ -407,7 +441,7 @@ def _cpu_window(kernel, pods, X, Yo, P, ib):
     return out[Yo, X].astype(np.int64)
 
 
-@pytest.mark.parametrize("win_id,P", WIN_CASES, ids=["%s-p%d" % c for c in WIN_CASES])
+@pytest.mark.parametrize("win_id,P", CPU_WIN_CASES, ids=["%s-p%d" % c for c in CPU_WIN_CASES])
 def test_window_cpu(built, win_id, P):
     """The oracle's restatement (1x, 2x) / the host-built four-limb loop: every certified sampled pixel equals the
     exact count."""
