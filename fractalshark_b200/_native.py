@@ -41,6 +41,9 @@ GPU_SYMBOLS = {
     "fs_test_cuda_is_working": (_U32, []),
     "fs_create": (_V, [_I32]),
     "fs_destroy": (None, [_V]),
+    "fs_create_group": (_V, [C.POINTER(C.c_int32), _U32]),
+    "fs_create_default": (_V, []),
+    "fs_device_count": (_U32, [_V]),
     "fs_initialize_memory": (_U32, [_V, _U32, _U32, _U32, _U32, _V, _U32, _U32, _U64, _I32]),
     "fs_initialize_perturb": (_U32, [_V, _U32, _I32, _I32, _U64, C.POINTER(FsOrbit), _I32, _U64, C.POINTER(FsOrbit),
                                      C.POINTER(FsLaReference)]),

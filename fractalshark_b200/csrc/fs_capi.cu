@@ -135,6 +135,17 @@ struct fs_renderer {
     int num_sms = 148;
     fs_done_callback cb = nullptr;
     void *cb_user = nullptr;
+    // device group (fs_create_group): member i renders shard (n, i) on its own device and every entry forwards to the
+    // members; member 0 is the lead.  Empty for handles of fs_create.
+    std::vector<fs_renderer *> members;
+    std::vector<cudaEvent_t> joins; // one per member, on its device: joins the member's stream into the lead's
+    Reduction *red_parts = nullptr; // on the lead: n member reductions + the frame's, for the compute and the display stream
+    // AA 3: the whole frame's iteration cells gathered on the lead, one buffer for the compute and one for the display
+    // stream.  cudaMalloc, not the stream-ordered pool: peer access (cudaDeviceEnablePeerAccess) covers it, so the members
+    // write their bands into it directly.  Allocated only while the group's antialiasing is 3.
+    void *gather[2] = {nullptr, nullptr};
+    size_t gather_bytes = 0;
+    cudaEvent_t lead_marks[2] = {nullptr, nullptr}; // on the lead's compute / display stream: what the lead has read so far
 };
 
 namespace {
@@ -846,7 +857,11 @@ template <class Pixel> uint32_t launch_direct_ext_pods(fs_renderer *r, const voi
                : launch_direct_ext<Pixel, uint32_t>(r, load_pod<Cd>(cx), load_pod<Cd>(cy), load_pod<Cd>(dx), load_pod<Cd>(dy), n_iter);
 }
 
-template <class IterT> uint32_t run_post(fs_renderer *r, uint64_t n_iter, cudaStream_t stream, bool colors = true) {
+// Colours and Min/Max/Sum of the 4-row bands b % shard_count == shard_index (1, 0: the whole frame) of r's buffers, or of
+// the iteration cells at `iters` (r's geometry) when given.
+template <class IterT>
+uint32_t run_post(fs_renderer *r, uint64_t n_iter, cudaStream_t stream, bool colors, uint32_t shard_count, uint32_t shard_index,
+                  const void *iters = nullptr) {
     same_carveout(r, reduction_init_kernel<IterT>);
     same_carveout(r, post_kernel<IterT, 1>);
     same_carveout(r, post_kernel<IterT, 2>);
@@ -855,8 +870,8 @@ template <class IterT> uint32_t run_post(fs_renderer *r, uint64_t n_iter, cudaSt
     reduction_init_kernel<IterT><<<1, 256, 0, stream>>>(r->red_dev); // 256 threads: same carve-out class as the render kernels
     const int pitch = (int)(r->w_block * NB_THREADS_W);
     const int grid = r->num_sms * 8;
-    const IterT *it = static_cast<const IterT *>(r->iter_buf);
-#define FS_POST_ARGS (it, pitch, r->color_buf, r->pal_dev, r->pal_iters, r->aux_depth, (int)r->color_w, (int)r->color_h, (IterT)n_iter, r->red_dev, (int)r->shard_count, (int)r->shard_index)
+    const IterT *it = static_cast<const IterT *>(iters ? iters : r->iter_buf);
+#define FS_POST_ARGS (it, pitch, r->color_buf, r->pal_dev, r->pal_iters, r->aux_depth, (int)r->color_w, (int)r->color_h, (IterT)n_iter, r->red_dev, (int)shard_count, (int)shard_index)
 #define FS_POST(AA)                                                                                                    \
     if (colors) post_kernel<IterT, AA, true><<<grid, 256, 0, stream>>> FS_POST_ARGS;                                    \
     else { same_carveout(r, post_kernel<IterT, AA, false>); post_kernel<IterT, AA, false><<<grid, 256, 0, stream>>> FS_POST_ARGS; }
@@ -924,6 +939,77 @@ __global__ void __launch_bounds__(256) dfma_peak_kernel(double *sink, int iters,
 void CUDART_CB done_trampoline(void *p) {
     fs_renderer *r = static_cast<fs_renderer *>(p);
     if (r->cb) r->cb(r->cb_user);
+}
+
+bool is_group(const fs_renderer *r) { return r && !r->members.empty(); }
+
+// Runs f on every member in order; the first non-zero status is the group's.
+template <class F> uint32_t each_member(fs_renderer *grp, F &&f) {
+    uint32_t first = 0;
+    for (fs_renderer *m : grp->members) {
+        const uint32_t rc = f(m);
+        if (rc && !first) first = rc;
+    }
+    return first;
+}
+
+// Makes `to`'s stream wait for everything enqueued so far on member i's stream `from`.
+cudaError_t join_member(fs_renderer *grp, size_t i, cudaStream_t from, cudaStream_t to) {
+    fs_renderer *m = grp->members[i];
+    DeviceGuard g(m->device);
+    cudaError_t err = cudaEventRecord(grp->joins[i], from);
+    if (err != cudaSuccess) return err;
+    return cudaStreamWaitEvent(to, grp->joins[i], 0);
+}
+
+
+void sync_members(fs_renderer *grp, bool display_too = false) {
+    for (fs_renderer *m : grp->members) {
+        if (!m->compute) continue;
+        DeviceGuard g(m->device);
+        cudaStreamSynchronize(m->compute);
+        if (display_too) cudaStreamSynchronize(m->display);
+    }
+}
+
+// Group state that needs the members' streams: the join events, the reduction parts on the lead and, at AA 3, the gather
+// buffers.  The combine kernel is loaded here for the reason preload_post_kernels gives.
+cudaError_t prepare_group(fs_renderer *grp) {
+    fs_renderer *lead = grp->members[0];
+    const size_t n = grp->members.size();
+    if (!grp->red_parts) {
+        grp->joins.assign(n, nullptr);
+        for (size_t i = 0; i < n; i++) {
+            DeviceGuard g(grp->members[i]->device);
+            cudaError_t err = cudaEventCreateWithFlags(&grp->joins[i], cudaEventDisableTiming);
+            if (err != cudaSuccess) return err;
+        }
+        DeviceGuard g(lead->device);
+        for (cudaEvent_t &e : grp->lead_marks) {
+            cudaError_t err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+            if (err != cudaSuccess) return err;
+        }
+        cudaFuncAttributes fa;
+        cudaFuncGetAttributes(&fa, reduction_combine_kernel);
+        cudaError_t err = cudaMalloc(&grp->red_parts, 2 * (n + 1) * sizeof(Reduction));
+        if (err != cudaSuccess) return err;
+    }
+    const size_t want = lead->aa == 3 ? lead->n_cu * lead->iter_bytes : 0;
+    if (grp->gather_bytes == want) return cudaSuccess;
+    sync_members(grp, true); // no member may still be writing into the old buffers
+    DeviceGuard g(lead->device);
+    for (void *&b : grp->gather) {
+        if (b) cudaFree(b);
+        b = nullptr;
+    }
+    grp->gather_bytes = 0;
+    for (void *&b : grp->gather) {
+        if (!want) break;
+        cudaError_t err = cudaMalloc(&b, want);
+        if (err != cudaSuccess) return err;
+    }
+    grp->gather_bytes = want;
+    return cudaSuccess;
 }
 
 } // namespace
@@ -1057,8 +1143,82 @@ fs_renderer *fs_create(int32_t device) {
     return r;
 }
 
+fs_renderer *fs_create_group(const int32_t *devices, uint32_t n) {
+    if (!devices || n == 0) return nullptr;
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess) { (void)cudaGetLastError(); return nullptr; }
+    for (uint32_t i = 0; i < n; i++)
+        if (devices[i] < 0 || devices[i] >= count) return nullptr;
+    if (n == 1) return fs_create(devices[0]);
+    fs_renderer *grp = new (std::nothrow) fs_renderer();
+    if (!grp) return nullptr;
+    grp->device = devices[0];
+    for (uint32_t i = 0; i < n; i++) {
+        fs_renderer *m = fs_create(devices[i]);
+        if (!m) { for (fs_renderer *k : grp->members) fs_destroy(k); grp->members.clear(); delete grp; return nullptr; }
+        m->shard_count = n;
+        m->shard_index = i;
+        grp->members.push_back(m);
+    }
+    // the members' bands meet on the lead (AA-3 colours, the reduction parts): direct over NVLink where the pair allows it.
+    // Peer access is per process and other groups may rely on it, so it is never disabled.
+    for (uint32_t i = 1; i < n; i++) {
+        const int a = devices[0], b = devices[i];
+        if (a == b) continue;
+        int ok = 0;
+        for (int k = 0; k < 2; k++) {
+            const int from = k ? b : a, to = k ? a : b;
+            if (cudaDeviceCanAccessPeer(&ok, from, to) != cudaSuccess || !ok) continue;
+            DeviceGuard g(from);
+            if (cudaDeviceEnablePeerAccess(to, 0) != cudaSuccess) (void)cudaGetLastError(); // e.g. already enabled
+        }
+    }
+    return grp;
+}
+
+fs_renderer *fs_create_default(void) {
+    const char *list = getenv("FS_GPU_DEVICES");
+    if (!list) return fs_create(0);
+    int32_t ids[64];
+    uint32_t n = 0;
+    const char *p = list;
+    for (;;) { // one or more digits per item, items separated by single commas
+        if (*p < '0' || *p > '9' || n == 64) return nullptr;
+        int64_t v = 0;
+        while (*p >= '0' && *p <= '9') {
+            v = v * 10 + (*p++ - '0');
+            if (v > INT32_MAX) return nullptr;
+        }
+        ids[n++] = (int32_t)v;
+        if (*p == '\0') break;
+        if (*p++ != ',') return nullptr;
+    }
+    return fs_create_group(ids, n);
+}
+
+uint32_t fs_device_count(const fs_renderer *r) { return !r ? 0 : is_group(r) ? (uint32_t)r->members.size() : 1; }
+
 void fs_destroy(fs_renderer *r) {
     if (!r) return;
+    if (is_group(r)) {
+        sync_members(r, true);
+        for (size_t i = 0; i < r->joins.size(); i++) {
+            DeviceGuard g(r->members[i]->device);
+            if (r->joins[i]) cudaEventDestroy(r->joins[i]);
+        }
+        {
+            DeviceGuard g(r->device);
+            for (cudaEvent_t e : r->lead_marks)
+                if (e) cudaEventDestroy(e);
+            for (void *b : r->gather)
+                if (b) cudaFree(b);
+            if (r->red_parts) cudaFree(r->red_parts);
+        }
+        // member 0 registered a result sink the others only map: it lets go of it last
+        for (size_t i = r->members.size(); i-- > 0;) fs_destroy(r->members[i]);
+        delete r;
+        return;
+    }
     DeviceGuard g(r->device);
     if (r->compute) {
         if (r->display) cudaStreamSynchronize(r->display);
@@ -1081,6 +1241,14 @@ void fs_destroy(fs_renderer *r) {
 uint32_t fs_initialize_memory(fs_renderer *r, uint32_t iter_bytes, uint32_t w, uint32_t h, uint32_t antialiasing,
                               const fs_color16 *pal, uint32_t pal_iters, uint32_t aux_depth, uint64_t pal_gen,
                               int32_t expected_reuse) {
+    if (is_group(r)) {
+        // a geometry change drops the result sink member 0 registered: no member may still be writing into it
+        if (r->members[0]->sink_dev) sync_members(r);
+        const uint32_t rc = each_member(r, [&](fs_renderer *m) {
+            return fs_initialize_memory(m, iter_bytes, w, h, antialiasing, pal, pal_iters, aux_depth, pal_gen, expected_reuse);
+        });
+        return rc ? rc : (uint32_t)prepare_group(r);
+    }
     if (!r || (iter_bytes != 4 && iter_bytes != 8)) return FS_ERROR_UNSUPPORTED;
     cudaError_t err = cudaSetDevice(r->device);
     if (err != cudaSuccess) return err;
@@ -1168,6 +1336,10 @@ uint32_t fs_initialize_memory(fs_renderer *r, uint32_t iter_bytes, uint32_t w, u
 uint32_t fs_initialize_perturb(fs_renderer *r, uint32_t iter_bytes, int32_t numeric1, int32_t pextras,
                                uint64_t generation1, const fs_orbit *perturb1, int32_t numeric2, uint64_t generation2,
                                const fs_orbit *perturb2, const fs_la_reference *la) {
+    if (is_group(r))
+        return each_member(r, [&](fs_renderer *m) {
+            return fs_initialize_perturb(m, iter_bytes, numeric1, pextras, generation1, perturb1, numeric2, generation2, perturb2, la);
+        });
     if (!r || !r->compute) return FS_ERROR_6_NO_ORBIT;
     DeviceGuard g(r->device);
     bool install_la = false;
@@ -1194,6 +1366,7 @@ uint32_t fs_initialize_perturb(fs_renderer *r, uint32_t iter_bytes, int32_t nume
 }
 
 void fs_clear_memory(fs_renderer *r) {
+    if (is_group(r)) { each_member(r, [](fs_renderer *m) { fs_clear_memory(m); return 0u; }); return; }
     if (!r || !r->compute) return;
     r->sink_filled = false;
     DeviceGuard g(r->device);
@@ -1204,6 +1377,10 @@ void fs_clear_memory(fs_renderer *r) {
 
 uint32_t fs_render(fs_renderer *r, uint32_t algorithm, int32_t numeric, const void *cx, const void *cy,
                    const void *dx, const void *dy, uint64_t n_iterations, int32_t iteration_precision) {
+    if (is_group(r))
+        return each_member(r, [&](fs_renderer *m) {
+            return fs_render(m, algorithm, numeric, cx, cy, dx, dy, n_iterations, iteration_precision);
+        });
     (void)algorithm;
     if (!r || !memory_initialized(r)) return 0; // GPU_Render.cu:626-628
     DeviceGuard g(r->device);
@@ -1247,6 +1424,10 @@ uint32_t fs_render(fs_renderer *r, uint32_t algorithm, int32_t numeric, const vo
 uint32_t fs_render_perturb_lav2(fs_renderer *r, uint32_t algorithm, int32_t numeric, int32_t mode, int32_t pextras,
                                 const void *cx, const void *cy, const void *dx, const void *dy, const void *center_x,
                                 const void *center_y, uint64_t n_iterations) {
+    if (is_group(r))
+        return each_member(r, [&](fs_renderer *m) {
+            return fs_render_perturb_lav2(m, algorithm, numeric, mode, pextras, cx, cy, dx, dy, center_x, center_y, n_iterations);
+        });
     (void)algorithm; (void)cx; (void)cy;
     if (!r || !memory_initialized(r)) return 0; // GPU_Render.cu:1007-1009
     DeviceGuard g(r->device);
@@ -1262,6 +1443,11 @@ uint32_t fs_render_perturb_bla(fs_renderer *r, uint32_t algorithm, int32_t numer
                                const fs_blas *blas, const void *cx, const void *cy, const void *dx, const void *dy,
                                const void *center_x, const void *center_y, uint64_t n_iterations,
                                int32_t iteration_precision) {
+    if (is_group(r))
+        return each_member(r, [&](fs_renderer *m) {
+            return fs_render_perturb_bla(m, algorithm, numeric, results, blas, cx, cy, dx, dy, center_x, center_y, n_iterations,
+                                         iteration_precision);
+        });
     (void)algorithm; (void)cx; (void)cy; (void)iteration_precision;
     if (!r || !memory_initialized(r)) return 0; // GPU_Render.cu:1454-1456
     if (!results || !blas) return FS_ERROR_6_NO_ORBIT;
@@ -1291,6 +1477,11 @@ uint32_t fs_render_perturb_bla_scaled(fs_renderer *r, uint32_t algorithm, int32_
                                       const fs_orbit *double_perturb, const fs_orbit *float_perturb, const void *cx,
                                       const void *cy, const void *dx, const void *dy, const void *center_x,
                                       const void *center_y, uint64_t n_iterations, int32_t iteration_precision) {
+    if (is_group(r))
+        return each_member(r, [&](fs_renderer *m) {
+            return fs_render_perturb_bla_scaled(m, algorithm, numeric, double_perturb, float_perturb, cx, cy, dx, dy, center_x,
+                                                center_y, n_iterations, iteration_precision);
+        });
     (void)algorithm; (void)cx; (void)cy; (void)iteration_precision;
     if (!r || !memory_initialized(r)) return 0; // GPU_Render.cu:1317-1319
     if (!double_perturb || !float_perturb) return FS_ERROR_6_NO_ORBIT;
@@ -1321,15 +1512,21 @@ static void request_yield_if_rendering(fs_renderer *r) {
     cudaMemcpyAsync(r->yield_quota, r->yield_src, sizeof(int), cudaMemcpyHostToDevice, r->display);
 }
 
+static cudaError_t copy_shard_bands(fs_renderer *r, void *iter_buffer, fs_color16 *color_buffer, cudaStream_t stream);
+static uint32_t group_render_current(fs_renderer *grp, uint64_t n_iterations, void *iter_buffer, fs_color16 *color_buffer,
+                                     fs_reduction *reduction_results, int32_t progressive);
+
 uint32_t fs_render_current(fs_renderer *r, uint64_t n_iterations, void *iter_buffer, fs_color16 *color_buffer,
                            fs_reduction *reduction_results, int32_t progressive) {
+    if (is_group(r)) return group_render_current(r, n_iterations, iter_buffer, color_buffer, reduction_results, progressive);
     if (!r || !memory_initialized(r)) return 0; // GPU_Render.cu:563-565
     DeviceGuard g(r->device);
     cudaStream_t stream = progressive ? r->display : r->compute;
     if (progressive) request_yield_if_rendering(r);
     // no colour buffer asked for: the reduction alone (the colour buffer on the device is then stale until a call that asks)
     const bool colors = color_buffer != nullptr;
-    uint32_t rc = r->iter_bytes == 8 ? run_post<uint64_t>(r, n_iterations, stream, colors) : run_post<uint32_t>(r, n_iterations, stream, colors);
+    uint32_t rc = r->iter_bytes == 8 ? run_post<uint64_t>(r, n_iterations, stream, colors, r->shard_count, r->shard_index)
+                                     : run_post<uint32_t>(r, n_iterations, stream, colors, r->shard_count, r->shard_index);
     if (rc) return rc;
     cudaError_t err = cudaSuccess;
     if (iter_buffer && !(r->sink_filled && iter_buffer == r->sink_host)) { // a filled sink already holds the frame
@@ -1353,6 +1550,7 @@ uint32_t fs_render_current(fs_renderer *r, uint64_t n_iterations, void *iter_buf
 // shard's cells only (post_kernel skips the others): the frame's reduction is min / max / sum over the shards'.
 uint32_t fs_render_current_shard(fs_renderer *r, uint64_t n_iterations, void *iter_buffer, fs_color16 *color_buffer,
                                  fs_reduction *reduction_results, int32_t progressive) {
+    if (is_group(r)) return FS_ERROR_UNSUPPORTED; // a group already is the sharding
     if (!r || !memory_initialized(r)) return 0;
     if (r->shard_count <= 1) return fs_render_current(r, n_iterations, iter_buffer, color_buffer, reduction_results, progressive);
     // an antialiasing cell must lie inside one 4-row band: 3x3 cells straddle bands, their colours would need other shards' rows
@@ -1361,19 +1559,37 @@ uint32_t fs_render_current_shard(fs_renderer *r, uint64_t n_iterations, void *it
     cudaStream_t stream = progressive ? r->display : r->compute;
     if (progressive) request_yield_if_rendering(r);
     const bool colors = color_buffer != nullptr;
-    uint32_t rc = r->iter_bytes == 8 ? run_post<uint64_t>(r, n_iterations, stream, colors) : run_post<uint32_t>(r, n_iterations, stream, colors);
+    uint32_t rc = r->iter_bytes == 8 ? run_post<uint64_t>(r, n_iterations, stream, colors, r->shard_count, r->shard_index)
+                                     : run_post<uint32_t>(r, n_iterations, stream, colors, r->shard_count, r->shard_index);
     if (rc) return rc;
+    cudaError_t err = copy_shard_bands(r, iter_buffer, color_buffer, stream);
+    if (err != cudaSuccess) return err;
+    if (reduction_results) {
+        err = cudaMemcpyAsync(reduction_results, r->red_dev, sizeof(Reduction), cudaMemcpyDefault, stream);
+        if (err != cudaSuccess) return err;
+    }
+    return 0;
+}
+
+// The shard's own 4-row bands of the iteration cells into the same positions of a whole-frame buffer (host, or another
+// renderer's device buffer): one strided 2-D copy.
+static cudaError_t copy_iter_bands(const fs_renderer *r, void *dst, cudaStream_t stream) {
+    const size_t row_bytes = (size_t)r->w_block * NB_THREADS_W * r->iter_bytes;
+    const size_t bands = (size_t)r->h_block * NB_THREADS_H / 4; // padded height is a multiple of 8
+    const size_t owned = (bands - r->shard_index + r->shard_count - 1) / r->shard_count;
+    const size_t first = (size_t)r->shard_index * 4 * row_bytes, stride = (size_t)r->shard_count * 4 * row_bytes;
+    if (!owned) return cudaSuccess;
+    return cudaMemcpy2DAsync((char *)dst + first, stride, (const char *)r->iter_buf + first, stride, 4 * row_bytes, owned,
+                             cudaMemcpyDefault, stream);
+}
+
+// The shard's own 4-row bands of the iteration cells (unless a filled sink already holds them) and, when color_buffer is
+// given, of the Color16 cells, into the same positions of whole-frame host buffers.
+static cudaError_t copy_shard_bands(fs_renderer *r, void *iter_buffer, fs_color16 *color_buffer, cudaStream_t stream) {
     cudaError_t err = cudaSuccess;
     if (iter_buffer && !(r->sink_filled && iter_buffer == r->sink_host)) {
-        const size_t row_bytes = (size_t)r->w_block * NB_THREADS_W * r->iter_bytes;
-        const size_t bands = (size_t)r->h_block * NB_THREADS_H / 4; // padded height is a multiple of 8
-        const size_t owned = (bands - r->shard_index + r->shard_count - 1) / r->shard_count;
-        const size_t first = (size_t)r->shard_index * 4 * row_bytes, stride = (size_t)r->shard_count * 4 * row_bytes;
-        if (owned) {
-            err = cudaMemcpy2DAsync((char *)iter_buffer + first, stride, (const char *)r->iter_buf + first, stride,
-                                    4 * row_bytes, owned, cudaMemcpyDefault, stream);
-            if (err != cudaSuccess) return err;
-        }
+        err = copy_iter_bands(r, iter_buffer, stream);
+        if (err != cudaSuccess) return err;
     }
     if (color_buffer) {
         // colour cells are stored un-padded (index oy * color_w + ox, AntialiasingKernel.cuh:3-71): the colour rows of one
@@ -1398,18 +1614,132 @@ uint32_t fs_render_current_shard(fs_renderer *r, uint64_t n_iterations, void *it
             if (err != cudaSuccess) return err;
         }
     }
+    return cudaSuccess;
+}
+
+// RenderCurrent of a device group: the bytes one renderer returns, assembled without a host synchronise.  Every member
+// copies its own iteration bands to the host over its own link.  AA 1/2/4: every member colours and reduces its own bands
+// (a cell never straddles two bands) and copies its colour bands; the members' reductions meet on the lead, where
+// reduction_combine_kernel makes the frame's.  AA 3: 3x3 cells straddle bands, so every member copies its iteration bands
+// into the lead's gather buffer (peer to peer) and the lead colours and reduces the whole frame from there.
+// Members write into lead-owned memory (reduction parts, gather buffer) only after the lead's stream has passed what it
+// had been given before this call, so result calls may follow each other without a synchronise in between.
+static uint32_t group_render_current(fs_renderer *grp, uint64_t n_iterations, void *iter_buffer, fs_color16 *color_buffer,
+                                     fs_reduction *reduction_results, int32_t progressive) {
+    fs_renderer *lead = grp->members[0];
+    if (!memory_initialized(lead) || !grp->red_parts) return 0;
+    const size_t n = grp->members.size();
+    const bool colors = color_buffer != nullptr;
+    const bool on_lead = lead->aa == 3;
+    const bool to_lead = colors || reduction_results; // anything beyond the iteration cells, which need no meeting point
+    const int slot = progressive ? 1 : 0;
+    auto stream_of = [&](fs_renderer *m) { return progressive ? m->display : m->compute; };
+    Reduction *parts = grp->red_parts + slot * (n + 1), *frame_red = parts + n;
+    void *gather = grp->gather[slot];
+    // fs_initialize_memory sizes the gather buffers; a call that failed on some member may have left them behind
+    if (on_lead && to_lead && (!gather || grp->gather_bytes != lead->n_cu * lead->iter_bytes)) return FS_ERROR_UNSUPPORTED;
+    cudaError_t err = cudaSuccess;
+    { // what the lead's stream has been given so far, including the reads of the previous result call on this stream
+        DeviceGuard g(lead->device);
+        err = cudaEventRecord(grp->lead_marks[slot], stream_of(lead));
+        if (err != cudaSuccess) return err;
+    }
+    for (size_t i = 0; i < n; i++) {
+        fs_renderer *m = grp->members[i];
+        DeviceGuard g(m->device);
+        const cudaStream_t s = stream_of(m);
+        if (progressive) request_yield_if_rendering(m);
+        if (!on_lead) {
+            const uint32_t rc = m->iter_bytes == 8 ? run_post<uint64_t>(m, n_iterations, s, colors, m->shard_count, m->shard_index)
+                                                   : run_post<uint32_t>(m, n_iterations, s, colors, m->shard_count, m->shard_index);
+            if (rc) return rc;
+        }
+        err = copy_shard_bands(m, iter_buffer, on_lead ? nullptr : color_buffer, s);
+        if (err != cudaSuccess) return err;
+        const bool writes_lead = on_lead ? to_lead : reduction_results != nullptr;
+        if (!writes_lead) continue;
+        if (i > 0) { // write only after the lead has read what the previous result call left there
+            err = cudaStreamWaitEvent(s, grp->lead_marks[slot], 0);
+            if (err != cudaSuccess) return err;
+        }
+        err = on_lead ? copy_iter_bands(m, gather, s)
+                      : cudaMemcpyPeerAsync(parts + i, lead->device, m->red_dev, m->device, sizeof(Reduction), s);
+        if (err != cudaSuccess) return err;
+        if (i > 0) {
+            err = join_member(grp, i, s, stream_of(lead));
+            if (err != cudaSuccess) return err;
+        }
+    }
+    DeviceGuard g(lead->device);
+    const cudaStream_t s = stream_of(lead);
+    if (on_lead) {
+        if (!to_lead) return 0;
+        const uint32_t rc = lead->iter_bytes == 8 ? run_post<uint64_t>(lead, n_iterations, s, colors, 1, 0, gather)
+                                                  : run_post<uint32_t>(lead, n_iterations, s, colors, 1, 0, gather);
+        if (rc) return rc;
+        if (color_buffer) {
+            err = cudaMemcpyAsync(color_buffer, lead->color_buf, lead->n_color_cu * sizeof(Color16), cudaMemcpyDefault, s);
+            if (err != cudaSuccess) return err;
+        }
+        if (reduction_results) {
+            err = cudaMemcpyAsync(reduction_results, lead->red_dev, sizeof(Reduction), cudaMemcpyDefault, s);
+            if (err != cudaSuccess) return err;
+        }
+        return 0;
+    }
+    if (color_buffer) { // the padding behind the colour cells, as fs_render_current copies it
+        const size_t cells = (size_t)lead->color_w * lead->color_h;
+        err = cudaMemcpyAsync(color_buffer + cells, lead->color_buf + cells, (lead->n_color_cu - cells) * sizeof(Color16),
+                              cudaMemcpyDefault, s);
+        if (err != cudaSuccess) return err;
+    }
     if (reduction_results) {
-        err = cudaMemcpyAsync(reduction_results, r->red_dev, sizeof(Reduction), cudaMemcpyDefault, stream);
+        auto k = reduction_combine_kernel;
+        same_carveout(lead, k);
+        k<<<1, 256, 0, s>>>(parts, (int)n, frame_red);
+        lead->launches++;
+        err = cudaGetLastError();
+        if (err != cudaSuccess) return err;
+        err = cudaMemcpyAsync(reduction_results, frame_red, sizeof(Reduction), cudaMemcpyDefault, s);
         if (err != cudaSuccess) return err;
     }
     return 0;
 }
 
-uint32_t fs_sync_compute_stream(fs_renderer *r) { DeviceGuard g(r->device); return cudaStreamSynchronize(r->compute); }
-uint32_t fs_sync_display_stream(fs_renderer *r) { DeviceGuard g(r->device); return cudaStreamSynchronize(r->display); }
-uint32_t fs_query_compute_stream(fs_renderer *r) { DeviceGuard g(r->device); return cudaStreamQuery(r->compute); }
+uint32_t fs_sync_compute_stream(fs_renderer *r) {
+    if (is_group(r)) return each_member(r, [](fs_renderer *m) { return fs_sync_compute_stream(m); });
+    DeviceGuard g(r->device);
+    return cudaStreamSynchronize(r->compute);
+}
+uint32_t fs_sync_display_stream(fs_renderer *r) {
+    if (is_group(r)) return each_member(r, [](fs_renderer *m) { return fs_sync_display_stream(m); });
+    DeviceGuard g(r->device);
+    return cudaStreamSynchronize(r->display);
+}
+uint32_t fs_query_compute_stream(fs_renderer *r) {
+    if (is_group(r)) {
+        uint32_t first = 0;
+        for (fs_renderer *m : r->members) {
+            const uint32_t rc = fs_query_compute_stream(m);
+            if (rc == cudaErrorNotReady) return rc;
+            if (rc && !first) first = rc;
+        }
+        return first;
+    }
+    DeviceGuard g(r->device);
+    return cudaStreamQuery(r->compute);
+}
 
 uint32_t fs_enqueue_compute_done_callback(fs_renderer *r, fs_done_callback fn, void *user) {
+    if (is_group(r)) { // once, after every member's render: the lead's compute stream joins the others, then calls back
+        if (!r->red_parts) return FS_ERROR_UNSUPPORTED;
+        fs_renderer *lead = r->members[0];
+        for (size_t i = 1; i < r->members.size(); i++) {
+            const cudaError_t err = join_member(r, i, r->members[i]->compute, lead->compute);
+            if (err != cudaSuccess) return err;
+        }
+        return fs_enqueue_compute_done_callback(lead, fn, user);
+    }
     DeviceGuard g(r->device);
     r->cb = fn;
     r->cb_user = user;
@@ -1429,17 +1759,28 @@ const char *fs_convert_error_to_string(uint32_t err) {
     }
 }
 
-uint32_t fs_get_width(const fs_renderer *r) { return r->width; }
-uint32_t fs_get_height(const fs_renderer *r) { return r->height; }
+uint32_t fs_get_width(const fs_renderer *r) { return is_group(r) ? r->members[0]->width : r->width; }
+uint32_t fs_get_height(const fs_renderer *r) { return is_group(r) ? r->members[0]->height : r->height; }
 
 uint32_t fs_set_shard(fs_renderer *r, uint32_t shard_count, uint32_t shard_index) {
-    if (!r || shard_count == 0 || shard_index >= shard_count) return FS_ERROR_UNSUPPORTED;
+    if (!r || is_group(r) || shard_count == 0 || shard_index >= shard_count) return FS_ERROR_UNSUPPORTED;
     r->shard_count = shard_count;
     r->shard_index = shard_index;
     return 0;
 }
 
 uint32_t fs_last_render_ms(fs_renderer *r, float *ms) {
+    if (is_group(r)) { // the frame is done when the slowest member is
+        float worst = 0.0f;
+        for (fs_renderer *m : r->members) {
+            float v = 0.0f;
+            const uint32_t rc = fs_last_render_ms(m, &v);
+            if (rc) return rc;
+            worst = v > worst ? v : worst;
+        }
+        *ms = worst;
+        return 0;
+    }
     if (!r || !r->timed) return cudaErrorNotReady;
     DeviceGuard g(r->device);
     cudaError_t err = cudaEventSynchronize(r->ev_stop);
@@ -1448,6 +1789,7 @@ uint32_t fs_last_render_ms(fs_renderer *r, float *ms) {
 }
 
 uint32_t fs_enable_step_counter(fs_renderer *r, int32_t enable) {
+    if (is_group(r)) return each_member(r, [&](fs_renderer *m) { return fs_enable_step_counter(m, enable); });
     if (!r || !r->compute) return FS_ERROR_UNSUPPORTED;
     DeviceGuard g(r->device);
     r->count_steps = enable != 0;
@@ -1455,6 +1797,17 @@ uint32_t fs_enable_step_counter(fs_renderer *r, int32_t enable) {
 }
 
 uint32_t fs_read_step_counter(fs_renderer *r, uint64_t *steps) {
+    if (is_group(r)) {
+        uint64_t total = 0;
+        for (fs_renderer *m : r->members) {
+            uint64_t v = 0;
+            const uint32_t rc = fs_read_step_counter(m, &v);
+            if (rc) return rc;
+            total += v;
+        }
+        *steps = total;
+        return 0;
+    }
     if (!r || !r->compute) return FS_ERROR_UNSUPPORTED;
     DeviceGuard g(r->device);
     unsigned long long v = 0;
@@ -1466,6 +1819,17 @@ uint32_t fs_read_step_counter(fs_renderer *r, uint64_t *steps) {
 }
 
 uint32_t fs_read_step_counters(fs_renderer *r, uint64_t *counters3) {
+    if (is_group(r) && counters3) {
+        uint64_t total[3] = {0, 0, 0};
+        for (fs_renderer *m : r->members) {
+            uint64_t v[3];
+            const uint32_t rc = fs_read_step_counters(m, v);
+            if (rc) return rc;
+            for (int k = 0; k < 3; k++) total[k] += v[k];
+        }
+        for (int k = 0; k < 3; k++) counters3[k] = total[k];
+        return 0;
+    }
     if (!r || !r->compute || !counters3) return FS_ERROR_UNSUPPORTED;
     DeviceGuard g(r->device);
     unsigned long long v[3] = {0, 0, 0};
@@ -1541,6 +1905,21 @@ uint32_t fs_measure_fp64_issue_peak(int32_t device, double *dfma_per_second) {
 // Streams the iteration buffer to the host while the render runs.  `host_iter_buffer` has the layout fs_render_current
 // fills; if it is not page-locked yet it is registered here (and unregistered when the sink is dropped).
 uint32_t fs_set_result_sink(fs_renderer *r, void *host_iter_buffer, uint64_t bytes) {
+    if (is_group(r)) {
+        // member 0 registers the frame (portable, mapped) and the others map the same registration on their devices.  It
+        // lets go of it last, after every member has stopped writing.
+        sync_members(r);
+        for (size_t i = r->members.size(); i-- > 0;) fs_set_result_sink(r->members[i], nullptr, 0);
+        if (!host_iter_buffer) return memory_initialized(r->members[0]) ? 0 : FS_ERROR_UNSUPPORTED;
+        for (size_t i = 0; i < r->members.size(); i++) {
+            const uint32_t rc = fs_set_result_sink(r->members[i], host_iter_buffer, bytes);
+            if (rc) {
+                for (size_t k = i; k-- > 0;) fs_set_result_sink(r->members[k], nullptr, 0);
+                return rc;
+            }
+        }
+        return 0;
+    }
     if (!r || !memory_initialized(r)) return FS_ERROR_UNSUPPORTED;
     DeviceGuard g(r->device);
     cudaStreamSynchronize(r->compute);
@@ -1567,6 +1946,7 @@ uint32_t fs_set_result_sink(fs_renderer *r, void *host_iter_buffer, uint64_t byt
 }
 
 uint32_t fs_set_split_at(fs_renderer *r, int32_t enable) {
+    if (is_group(r)) return each_member(r, [&](fs_renderer *m) { return fs_set_split_at(m, enable); });
     if (!r) return FS_ERROR_UNSUPPORTED;
     r->split_at = enable != 0;
     return 0;
@@ -1599,12 +1979,14 @@ uint32_t fs_debug_pool_counters(uint64_t *out16) {
 #endif
 
 uint32_t fs_set_at_cycle_detection(fs_renderer *r, int32_t enable) {
+    if (is_group(r)) return each_member(r, [&](fs_renderer *m) { return fs_set_at_cycle_detection(m, enable); });
     if (!r) return FS_ERROR_UNSUPPORTED;
     r->at_cycle = enable != 0;
     return 0;
 }
 
 uint32_t fs_set_la_step2(fs_renderer *r, int32_t enable) {
+    if (is_group(r)) return each_member(r, [&](fs_renderer *m) { return fs_set_la_step2(m, enable); });
     if (!r) return FS_ERROR_UNSUPPORTED;
     r->use_la2 = enable != 0;
     return 0;
@@ -1633,18 +2015,27 @@ uint32_t fs_selftest_numeric_op(int32_t device, uint32_t op, const void *a, cons
 }
 
 uint32_t fs_set_pool_kernel(fs_renderer *r, int32_t enable) {
+    if (is_group(r)) return each_member(r, [&](fs_renderer *m) { return fs_set_pool_kernel(m, enable); });
     if (!r) return FS_ERROR_UNSUPPORTED;
     r->use_pool = enable != 0;
     return 0;
 }
 
 uint32_t fs_set_scaled_steps(fs_renderer *r, int32_t enable) {
+    if (is_group(r)) return each_member(r, [&](fs_renderer *m) { return fs_set_scaled_steps(m, enable); });
     if (!r) return FS_ERROR_UNSUPPORTED;
     r->use_scaled = enable != 0;
     return 0;
 }
 
-void *fs_device_iter_buffer(fs_renderer *r) { return r ? r->iter_buf : nullptr; }
-uint64_t fs_kernel_launch_count(const fs_renderer *r) { return r ? r->launches : 0; }
+void *fs_device_iter_buffer(fs_renderer *r) { return is_group(r) ? r->members[0]->iter_buf : r ? r->iter_buf : nullptr; }
+uint64_t fs_kernel_launch_count(const fs_renderer *r) {
+    if (is_group(r)) {
+        uint64_t total = 0;
+        for (const fs_renderer *m : r->members) total += m->launches;
+        return total;
+    }
+    return r ? r->launches : 0;
+}
 
 } // extern "C"

@@ -86,4 +86,17 @@ __global__ void __launch_bounds__(256) post_kernel(const IterT *__restrict__ ite
     }
 }
 
+// Device groups: the frame's Min/Max/Sum from the members' reductions of their own bands, on the lead device, so the
+// result call stays enqueue-only.  A member that owns no cell contributes the neutral {IterT max, 0, 0}.
+__global__ void __launch_bounds__(256) reduction_combine_kernel(const Reduction *__restrict__ parts, int n, Reduction *out) {
+    if (threadIdx.x != 0) return;
+    Reduction r = parts[0];
+    for (int i = 1; i < n; i++) {
+        r.Min = parts[i].Min < r.Min ? parts[i].Min : r.Min;
+        r.Max = parts[i].Max > r.Max ? parts[i].Max : r.Max;
+        r.Sum += parts[i].Sum;
+    }
+    *out = r;
+}
+
 } // namespace fs

@@ -27,11 +27,17 @@ def _buf(b: bytes):
 
 
 class GPURenderer:
-    def __init__(self, device: int = 0):
+    def __init__(self, device: int = 0, devices=None):
+        """``devices``: a list of device ids makes a device group (``fs_create_group``): one handle whose every call
+        renders the frame on all of them, member i rendering the 4-row bands b % n == i; ids may repeat."""
         self._lib = N.gpu_lib()
-        self._h = self._lib.fs_create(device)
+        if devices is None:
+            self._h = self._lib.fs_create(device)
+        else:
+            ids = (C.c_int32 * len(devices))(*devices)
+            self._h = self._lib.fs_create_group(ids, len(devices))
         if not self._h:
-            raise MemoryError("fs_create failed")
+            raise MemoryError("fs_create failed" if devices is None else f"fs_create_group({list(devices)}) failed")
         self._iter_bytes = 4
         self._keep = []  # host buffers borrowed by in-flight async copies
         self._cb = None
@@ -272,6 +278,10 @@ class GPURenderer:
     def SetPoolKernel(self, enable: bool = True) -> int:
         """A/B switch of the HDRx32 LAv2 path: lane-refill kernel (default) or one tile per warp (same results)."""
         return int(self._lib.fs_set_pool_kernel(self._h, int(enable)))
+
+    def DeviceCount(self) -> int:
+        """1 for a single renderer, n for a device group."""
+        return int(self._lib.fs_device_count(self._h))
 
     def DeviceIterBuffer(self) -> int:
         return int(self._lib.fs_device_iter_buffer(self._h) or 0)

@@ -95,6 +95,23 @@ uint32_t fs_test_cuda_is_working(void);                        /* GPURenderer::T
 fs_renderer *fs_create(int32_t device);                        /* GPURenderer()  (reference: always device 0)       */
 void fs_destroy(fs_renderer *r);                               /* ~GPURenderer()                                    */
 
+/* Device group (no reference counterpart): one handle that renders every frame on n devices.  Member i runs on
+ * devices[i] and renders the 4-row bands b % n == i (the fs_set_shard rule); ids may repeat ({0, 0, 0} is three shards
+ * on one GPU).  Every entry accepts the handle: uploads, clears, setters and render calls go to every member (render calls
+ * enqueue on all of them from the calling thread; status = the first non-zero member status), fs_render_current
+ * returns the same bytes a single renderer returns (iteration cells, colours at every antialiasing, Min/Max/Sum) and
+ * stays enqueue-only (result calls may follow each other without a synchronise), the done callback runs once after
+ * every member's render, step counters and launch counts are summed, fs_last_render_ms is the slowest member's, fs_get_width/height and fs_device_iter_buffer are member 0's.
+ * fs_set_shard and fs_render_current_shard return FS_ERROR_UNSUPPORTED.  NULL for n == 0, an id outside
+ * [0, device count) or an allocation failure; n == 1 is fs_create(devices[0]). */
+fs_renderer *fs_create_group(const int32_t *devices, uint32_t n);
+/* fs_create(0) when the environment variable FS_GPU_DEVICES is unset; else the group on the listed devices (decimal ids
+ * separated by commas, e.g. "0,1,2,3").  NULL, before any CUDA call, for a malformed list: an empty item, a character
+ * other than a digit or a comma, or more than 64 ids. */
+fs_renderer *fs_create_default(void);
+/* 1 for handles of fs_create, n for groups. */
+uint32_t fs_device_count(const fs_renderer *r);
+
 /* GPURenderer::InitializeMemory<IterType>  GPU_Render.h:91-100 ; iter_bytes = sizeof(IterType) (4|8) */
 uint32_t fs_initialize_memory(fs_renderer *r, uint32_t iter_bytes, uint32_t w, uint32_t h, uint32_t antialiasing,
                               const fs_color16 *pal_interleaved, uint32_t pal_iters, uint32_t palette_aux_depth,
