@@ -50,6 +50,8 @@ GPU_SYMBOLS = {
     "fs_clear_memory": (None, [_V]),
     "fs_render": (_U32, [_V, _U32, _I32, _V, _V, _V, _V, _U64, _I32]),
     "fs_render_perturb_lav2": (_U32, [_V, _U32, _I32, _I32, _I32, _V, _V, _V, _V, _V, _V, _U64]),
+    "fs_render_perturb_lav2_frames": (_U32, [_V, _U32, _I32, _I32, _I32, _U32, _V, _V, _V, _V, _V, _V, _U64]),
+    "fs_select_frame": (_U32, [_V, _U32]),
     "fs_render_perturb_bla": (_U32, [_V, _U32, _I32, C.POINTER(FsOrbit), C.POINTER(FsBlas), _V, _V, _V, _V, _V, _V,
                                      _U64, _I32]),
     "fs_render_perturb_bla_scaled": (_U32, [_V, _U32, _I32, C.POINTER(FsOrbit), C.POINTER(FsOrbit), _V, _V, _V, _V,
@@ -83,6 +85,7 @@ GPU_SYMBOLS = {
 
 HOST_SYMBOLS = {
     "fsh_view_create": (_V, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p, _U32, _U32, _U32, _I32]),
+    "fsh_view_zoom": (_V, [_V, C.c_char_p]),
     "fsh_view_destroy": (None, [_V]),
     "fsh_view_precision_bits": (_U32, [_V]),
     "fsh_view_coords": (_I32, [_V, _I32, _V, _V, _V, _V, _V, _V]),

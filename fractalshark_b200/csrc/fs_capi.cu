@@ -146,6 +146,13 @@ struct fs_renderer {
     void *gather[2] = {nullptr, nullptr};
     size_t gather_bytes = 0;
     cudaEvent_t lead_marks[2] = {nullptr, nullptr}; // on the lead's compute / display stream: what the lead has read so far
+    // zoom batches (fs_render_perturb_lav2_frames): frame 0 renders into iter_buf, frames 1..n-1 into the frame stack, which
+    // has iter_buf's layout per frame and comes from the same allocator, so every result path treats a stack frame as it
+    // treats iter_buf.  Result calls read frame `selected` (fs_select_frame) of the last render's `n_frames`.
+    void *frame_stack = nullptr;
+    uint32_t stack_frames = 0;
+    uint32_t n_frames = 0, selected = 0; // n_frames = 0: nothing rendered since the buffers were allocated
+    DeviceBlob frame_recs;               // the batch's Lav2Frame records
 };
 
 namespace {
@@ -217,6 +224,11 @@ void drop_sink(fs_renderer *r) {
 void reset_buffers(fs_renderer *r) {
     drop_sink(r);
     free_blob(r, r->at_state);
+    free_blob(r, r->frame_recs);
+    if (r->frame_stack) cudaFreeAsync(r->frame_stack, r->compute);
+    r->frame_stack = nullptr;
+    r->stack_frames = 0;
+    r->n_frames = r->selected = 0;
     if (r->iter_buf) cudaFreeAsync(r->iter_buf, r->compute);
     if (r->red_dev) cudaFreeAsync(r->red_dev, r->compute);
     if (r->color_buf) cudaFreeAsync(r->color_buf, r->compute);
@@ -226,6 +238,12 @@ void reset_buffers(fs_renderer *r) {
 }
 
 bool memory_initialized(const fs_renderer *r) { return r->iter_buf && r->red_dev && r->color_buf; }
+
+// The iteration cells every result call reads: frame `selected` of the last render (frame 0 = iter_buf).
+void *selected_iter_buf(const fs_renderer *r) {
+    if (r->selected == 0) return r->iter_buf;
+    return static_cast<char *>(r->frame_stack) + (size_t)(r->selected - 1) * r->n_cu * r->iter_bytes;
+}
 
 template <class T> T load_pod_early(const void *p) {
     T v;
@@ -540,6 +558,8 @@ TileQueue render_queue(fs_renderer *r) {
 
 void begin_render(fs_renderer *r, bool streams_to_sink = false) {
     r->sink_filled = streams_to_sink && r->sink_dev != nullptr; // any other render makes the host copy stale
+    r->n_frames = 1; // a zoom batch sets its own count after this
+    r->selected = 0;
     // tile counter and yield quota are adjacent words: one memset
     cudaMemsetAsync(r->tile_counter, 0, 2 * sizeof(unsigned int), r->compute);
     r->yield_requested = false;
@@ -558,8 +578,10 @@ template <class T> T load_pod(const void *p) {
     return v;
 }
 
+// Arguments of the LAv2 kernels for r's orbit, tables, geometry and switches; `have_la`: the LA table matches the orbit.
 template <class Num, class IterT>
-uint32_t launch_lav2(fs_renderer *r, int mode, const void *dx, const void *dy, const void *cx, const void *cy, uint64_t n_iter) {
+Lav2Args<Num, IterT> lav2_args(fs_renderer *r, const void *dx, const void *dy, const void *cx, const void *cy, uint64_t n_iter,
+                               bool &have_la) {
     using Real = typename Num::Real;
     Lav2Args<Num, IterT> A;
     memset(&A, 0, sizeof(A));
@@ -567,7 +589,7 @@ uint32_t launch_lav2(fs_renderer *r, int mode, const void *dx, const void *dy, c
     A.orbit = r->orbit1.data.ptr;
     A.orbit_fast = r->use_scaled ? r->orbit1.fast.ptr : nullptr;
     A.orbit_count = (IterT)r->orbit1.uncompressed;
-    const bool have_la = r->la.present && r->la.numeric == r->orbit1.numeric && r->la.iter_bytes == sizeof(IterT);
+    have_la = r->la.present && r->la.numeric == r->orbit1.numeric && r->la.iter_bytes == sizeof(IterT);
     if (have_la) {
         A.las = static_cast<const LaRec<Num, IterT> *>(r->la.las.ptr);
         A.stages = static_cast<const StageRec<IterT> *>(r->la.stages.ptr);
@@ -592,6 +614,13 @@ uint32_t launch_lav2(fs_renderer *r, int mode, const void *dx, const void *dy, c
     A.at_cycle = r->at_cycle ? 1 : 0;
     A.queue = render_queue(r);
     A.step_counter = r->count_steps ? r->step_counter : nullptr;
+    return A;
+}
+
+template <class Num, class IterT>
+uint32_t launch_lav2(fs_renderer *r, int mode, const void *dx, const void *dy, const void *cx, const void *cy, uint64_t n_iter) {
+    bool have_la = false;
+    Lav2Args<Num, IterT> A = lav2_args<Num, IterT>(r, dx, dy, cx, cy, n_iter, have_la);
     const bool count = r->count_steps;
     // two-launch form (AT, then everything else) for the float+exponent binary32 type when the table has an AT block
     if constexpr (Num::kHdr && !Num::kDf && sizeof(typename Num::Mant) == 4) {
@@ -682,6 +711,70 @@ uint32_t launch_lav2(fs_renderer *r, int mode, const void *dx, const void *dy, c
     default: return FS_ERROR_UNSUPPORTED;
     }
 #undef FS_LAUNCH_LAV2
+    return end_render(r);
+}
+
+// A zoom batch: n_frames frames of r's orbit and tables in one launch of lav2_kernel<..., Frames = true>.  `dx` ... `cy`
+// hold n_frames PODs each.  The batch always runs the fused tile kernel: the split-AT, lane-refill and probe-order
+// switches of launch_lav2 only change how a single frame is scheduled, never its cells, so a batch ignores them.
+template <class Num, class IterT>
+uint32_t launch_lav2_frames(fs_renderer *r, int mode, uint32_t n_frames, const void *dx, const void *dy, const void *cx,
+                            const void *cy, uint64_t n_iter) {
+    using Real = typename Num::Real;
+    using Frame = Lav2Frame<Num, IterT>;
+    if (mode != FS_LAV2_FULL && mode != FS_LAV2_PO && mode != FS_LAV2_LAO) return FS_ERROR_UNSUPPORTED;
+    const uint64_t bands = ((r->height + 3) / 4 + r->shard_count - 1 - r->shard_index) / r->shard_count;
+    if ((r->width + 7) / 8 * bands * n_frames >= (1ull << 31)) return FS_ERROR_UNSUPPORTED; // tickets are 32-bit
+    const size_t frame_bytes = r->n_cu * r->iter_bytes;
+    if (r->stack_frames < n_frames - 1) {
+        // a progressive RenderCurrent may still be reading a frame of the old stack on the display stream
+        cudaStreamSynchronize(r->display);
+        if (r->frame_stack) cudaFreeAsync(r->frame_stack, r->compute);
+        r->frame_stack = nullptr;
+        r->stack_frames = 0;
+        cudaError_t err = cudaMallocAsync(&r->frame_stack, (n_frames - 1) * frame_bytes, r->compute);
+        if (err != cudaSuccess) return err;
+        err = cudaMemsetAsync(r->frame_stack, 0, (n_frames - 1) * frame_bytes, r->compute);
+        if (err != cudaSuccess) return err;
+        r->stack_frames = n_frames - 1;
+        cudaEventRecord(r->ev_alloc, r->compute);
+        cudaStreamWaitEvent(r->display, r->ev_alloc, 0);
+    }
+    const size_t recs_bytes = (size_t)FS_MAX_FRAMES * sizeof(Frame);
+    if (r->frame_recs.bytes < recs_bytes) {
+        free_blob(r, r->frame_recs);
+        cudaError_t err = cudaMallocAsync(&r->frame_recs.ptr, recs_bytes, r->compute);
+        if (err != cudaSuccess) return err;
+        r->frame_recs.bytes = recs_bytes;
+    }
+    Frame recs[FS_MAX_FRAMES];
+    for (uint32_t f = 0; f < n_frames; f++) {
+        recs[f].dx = load_pod<Real>(static_cast<const char *>(dx) + f * sizeof(Real));
+        recs[f].dy = load_pod<Real>(static_cast<const char *>(dy) + f * sizeof(Real));
+        recs[f].centerX = load_pod<Real>(static_cast<const char *>(cx) + f * sizeof(Real));
+        recs[f].centerY = load_pod<Real>(static_cast<const char *>(cy) + f * sizeof(Real));
+        recs[f].out = static_cast<IterT *>(f == 0 ? r->iter_buf : static_cast<char *>(r->frame_stack) + (f - 1) * frame_bytes);
+    }
+    cudaError_t err = cudaMemcpyAsync(r->frame_recs.ptr, recs, n_frames * sizeof(Frame), cudaMemcpyHostToDevice, r->compute);
+    if (err != cudaSuccess) return err;
+    bool have_la = false;
+    Lav2Args<Num, IterT> A = lav2_args<Num, IterT>(r, dx, dy, cx, cy, n_iter, have_la);
+    A.out = nullptr;
+    A.sink = nullptr;
+    A.frames = static_cast<const Frame *>(r->frame_recs.ptr);
+    A.n_frames = n_frames;
+    begin_render(r);
+    r->n_frames = n_frames;
+    const bool count = r->count_steps;
+#define FS_LAUNCH_FRAMES(MODE)                                                                                         \
+    if (count) { auto k = lav2_kernel<Num, IterT, MODE, true, AtPhase::Fused, true>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); } \
+    else { auto k = lav2_kernel<Num, IterT, MODE, false, AtPhase::Fused, true>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); }
+    switch (mode) {
+    case FS_LAV2_FULL: FS_LAUNCH_FRAMES(Lav2Mode::Full) break;
+    case FS_LAV2_PO: FS_LAUNCH_FRAMES(Lav2Mode::PO) break;
+    default: FS_LAUNCH_FRAMES(Lav2Mode::LAO) break;
+    }
+#undef FS_LAUNCH_FRAMES
     return end_render(r);
 }
 
@@ -870,7 +963,7 @@ uint32_t run_post(fs_renderer *r, uint64_t n_iter, cudaStream_t stream, bool col
     reduction_init_kernel<IterT><<<1, 256, 0, stream>>>(r->red_dev); // 256 threads: same carve-out class as the render kernels
     const int pitch = (int)(r->w_block * NB_THREADS_W);
     const int grid = r->num_sms * 8;
-    const IterT *it = static_cast<const IterT *>(iters ? iters : r->iter_buf);
+    const IterT *it = static_cast<const IterT *>(iters ? iters : selected_iter_buf(r));
 #define FS_POST_ARGS (it, pitch, r->color_buf, r->pal_dev, r->pal_iters, r->aux_depth, (int)r->color_w, (int)r->color_h, (IterT)n_iter, r->red_dev, (int)shard_count, (int)shard_index)
 #define FS_POST(AA)                                                                                                    \
     if (colors) post_kernel<IterT, AA, true><<<grid, 256, 0, stream>>> FS_POST_ARGS;                                    \
@@ -1371,6 +1464,7 @@ void fs_clear_memory(fs_renderer *r) {
     r->sink_filled = false;
     DeviceGuard g(r->device);
     if (r->iter_buf) cudaMemsetAsync(r->iter_buf, 0, r->n_cu * r->iter_bytes, r->compute);
+    if (r->frame_stack) cudaMemsetAsync(r->frame_stack, 0, r->stack_frames * r->n_cu * r->iter_bytes, r->compute);
     if (r->red_dev) cudaMemsetAsync(r->red_dev, 0, r->iter_bytes, r->compute);
     if (r->color_buf) cudaMemsetAsync(r->color_buf, 0, r->n_color_cu * sizeof(Color16), r->compute);
 }
@@ -1437,6 +1531,36 @@ uint32_t fs_render_perturb_lav2(fs_renderer *r, uint32_t algorithm, int32_t nume
     return dispatch_num_iter(numeric, r->iter_bytes, [&](auto num, auto it) -> uint32_t {
         return launch_lav2<decltype(num), decltype(it)>(r, mode, dx, dy, center_x, center_y, n_iterations);
     });
+}
+
+uint32_t fs_render_perturb_lav2_frames(fs_renderer *r, uint32_t algorithm, int32_t numeric, int32_t mode, int32_t pextras,
+                                       uint32_t n_frames, const void *cx, const void *cy, const void *dx, const void *dy,
+                                       const void *center_x, const void *center_y, uint64_t n_iterations) {
+    if (!r || n_frames == 0 || n_frames > FS_MAX_FRAMES || !dx || !dy || !center_x || !center_y) return FS_ERROR_UNSUPPORTED;
+    if (is_group(r))
+        return each_member(r, [&](fs_renderer *m) {
+            return fs_render_perturb_lav2_frames(m, algorithm, numeric, mode, pextras, n_frames, cx, cy, dx, dy, center_x,
+                                                 center_y, n_iterations);
+        });
+    (void)algorithm; (void)cx; (void)cy;
+    if (!memory_initialized(r)) return 0; // as fs_render_perturb_lav2
+    DeviceGuard g(r->device);
+    if (!r->orbit1.valid || r->orbit1.numeric != numeric || r->orbit1.pextras != pextras) return FS_ERROR_6_NO_ORBIT;
+    if (pextras != FS_PEXTRAS_DISABLE && pextras != FS_PEXTRAS_SIMPLE_COMPRESSION) return FS_ERROR_UNSUPPORTED;
+    return dispatch_num_iter(numeric, r->iter_bytes, [&](auto num, auto it) -> uint32_t {
+        return launch_lav2_frames<decltype(num), decltype(it)>(r, mode, n_frames, dx, dy, center_x, center_y, n_iterations);
+    });
+}
+
+uint32_t fs_select_frame(fs_renderer *r, uint32_t k) {
+    if (is_group(r)) {
+        for (fs_renderer *m : r->members) // all members rendered the same batch: refuse before any of them changes
+            if (k >= m->n_frames) return FS_ERROR_UNSUPPORTED;
+        return each_member(r, [&](fs_renderer *m) { return fs_select_frame(m, k); });
+    }
+    if (!r || k >= r->n_frames) return FS_ERROR_UNSUPPORTED;
+    r->selected = k;
+    return 0;
 }
 
 uint32_t fs_render_perturb_bla(fs_renderer *r, uint32_t algorithm, int32_t numeric, const fs_orbit *results,
@@ -1530,7 +1654,7 @@ uint32_t fs_render_current(fs_renderer *r, uint64_t n_iterations, void *iter_buf
     if (rc) return rc;
     cudaError_t err = cudaSuccess;
     if (iter_buffer && !(r->sink_filled && iter_buffer == r->sink_host)) { // a filled sink already holds the frame
-        err = cudaMemcpyAsync(iter_buffer, r->iter_buf, r->n_cu * r->iter_bytes, cudaMemcpyDefault, stream);
+        err = cudaMemcpyAsync(iter_buffer, selected_iter_buf(r), r->n_cu * r->iter_bytes, cudaMemcpyDefault, stream);
         if (err != cudaSuccess) return err;
     }
     if (color_buffer) {
@@ -1579,7 +1703,7 @@ static cudaError_t copy_iter_bands(const fs_renderer *r, void *dst, cudaStream_t
     const size_t owned = (bands - r->shard_index + r->shard_count - 1) / r->shard_count;
     const size_t first = (size_t)r->shard_index * 4 * row_bytes, stride = (size_t)r->shard_count * 4 * row_bytes;
     if (!owned) return cudaSuccess;
-    return cudaMemcpy2DAsync((char *)dst + first, stride, (const char *)r->iter_buf + first, stride, 4 * row_bytes, owned,
+    return cudaMemcpy2DAsync((char *)dst + first, stride, (const char *)selected_iter_buf(r) + first, stride, 4 * row_bytes, owned,
                              cudaMemcpyDefault, stream);
 }
 
@@ -2028,7 +2152,9 @@ uint32_t fs_set_scaled_steps(fs_renderer *r, int32_t enable) {
     return 0;
 }
 
-void *fs_device_iter_buffer(fs_renderer *r) { return is_group(r) ? r->members[0]->iter_buf : r ? r->iter_buf : nullptr; }
+void *fs_device_iter_buffer(fs_renderer *r) {
+    return is_group(r) ? selected_iter_buf(r->members[0]) : r && r->iter_buf ? selected_iter_buf(r) : nullptr;
+}
 uint64_t fs_kernel_launch_count(const fs_renderer *r) {
     if (is_group(r)) {
         uint64_t total = 0;

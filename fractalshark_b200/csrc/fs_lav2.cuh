@@ -110,6 +110,12 @@ template <class Num, class IterT> struct AtDev {
     typename Num::Cplx InvZCoeff;
 };
 
+// One frame of a zoom batch (fs_render_perturb_lav2_frames): what differs between frames that share the orbit and tables.
+template <class Num, class IterT> struct Lav2Frame {
+    typename Num::Real dx, dy, centerX, centerY;
+    IterT *out; // this frame's iteration buffer, same padded layout as Lav2Args::out
+};
+
 template <class Num, class IterT> struct Lav2Args {
     IterT *out;              // iteration buffer, row pitch = roundup16(width)
     const void *orbit;       // reference-layout orbit elements (GPU_ReferenceIter.h:119-125)
@@ -133,6 +139,8 @@ template <class Num, class IterT> struct Lav2Args {
     const unsigned int *order;        // optional: queue position -> tile ticket (lav2_probe_kernel: expensive tiles first)
     int at_cycle;                     // 1: cycle detection in the AT shortcut (CycleWatch), 0: every pass is executed
     IterT *sink;                      // optional mapped host copy of `out` (fs_set_result_sink): finished pixels stream out over PCIe
+    const Lav2Frame<Num, IterT> *frames; // lav2_kernel<..., Frames = true>: n_frames records; dx, dy, centerX, centerY, out unused
+    unsigned int n_frames;
 };
 
 // How a launch treats the AT shortcut.  Fused = one launch does everything (the reference's structure).  On deep views
@@ -642,29 +650,46 @@ FS_D void lav2_stages_v2(const Lav2Args<NumHdr<float>, uint32_t> &A, const HdrC<
     }
 }
 
-template <class Num, class IterT, Lav2Mode Mode, bool Count, AtPhase Phase = AtPhase::Fused>
+// Frames = true renders a zoom batch: A.n_frames frames that share the orbit and the tables, each with its own pixel
+// spacing, centre offset and iteration buffer (A.frames).  The queue hands out n_frames x n_tiles tickets, frame-major,
+// so the SMs that finish frame k's cheap tiles pick up frame k + 1's while frame k's expensive tiles still run: only the
+// last frame's tail is left at the end of the launch.  Tiles of every frame keep the centre-out order and the shard rule.
+// No result sink, no probe order.
+template <class Num, class IterT, Lav2Mode Mode, bool Count, AtPhase Phase = AtPhase::Fused, bool Frames = false>
 __global__ void FS_LAV2_BOUNDS(Num) lav2_kernel(const Lav2Args<Num, IterT> A) {
     using Real = typename Num::Real;
     using Cplx = typename Num::Cplx;
+    static_assert(!Frames || Phase == AtPhase::Fused, "zoom batches run the fused kernel");
 
     const int lane = threadIdx.x & 31;
     const int tiles_x = (A.width + 7) >> 3;
     const int tiles_y = (((A.height + 3) >> 2) - A.shard_index + A.shard_count - 1) / A.shard_count;
     const unsigned int n_tiles = (unsigned int)tiles_x * (unsigned int)tiles_y;
+    const unsigned int n_tickets = Frames ? n_tiles * A.n_frames : n_tiles;
     unsigned long long steps = 0, steps_at = 0, steps_la = 0;
 
     TileCursor cursor;
     tile_queue_begin(cursor);
     for (;;) {
         unsigned int tile;
-        if (!next_tile(A.queue, cursor, n_tiles, tile)) break;
+        if (!next_tile(A.queue, cursor, n_tickets, tile)) break;
+        Real fdx = A.dx, fdy = A.dy, fcx = A.centerX, fcy = A.centerY;
+        if constexpr (Frames) {
+            const unsigned int frame = tile / n_tiles; // warp-uniform
+            tile -= frame * n_tiles;
+            const Lav2Frame<Num, IterT> *fr = A.frames + frame;
+            fdx = fr->dx;
+            fdy = fr->dy;
+            fcx = fr->centerX;
+            fcy = fr->centerY;
+        }
 
 #ifdef FS_TILE_TIMING
         const long long fs_t0 = clock64();
         unsigned long long fs_g0;
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(fs_g0));
 #endif
-        if (A.order) {
+        if (!Frames && A.order) {
             // two lists filled by lav2_probe_kernel, each in ticket (centre-out) order: expensive tiles, then the rest
             const unsigned int n_first = *(const volatile unsigned int *)(A.order + 2 * (size_t)n_tiles);
             tile = tile < n_first ? __ldg(A.order + tile) : __ldg(A.order + n_tiles + (tile - n_first));
@@ -679,8 +704,8 @@ __global__ void FS_LAV2_BOUNDS(Num) lav2_kernel(const Lav2Args<Num, IterT> A) {
         IterT iter = 0;
         IterT RefIteration = 0;
         // LAKernel.cuh:41-42 (no reduction of the deltas here)
-        const Real dcX = Num::delta_x(A.dx, X, A.centerX);
-        const Real dcY = Num::delta_y(A.dy, Y, A.centerY);
+        const Real dcX = Num::delta_x(fdx, X, fcx);
+        const Real dcY = Num::delta_y(fdy, Y, fcy);
         const Cplx dc = Num::c_make(dcX, dcY);
         Cplx dz = Num::c_zero();
 
@@ -725,8 +750,14 @@ __global__ void FS_LAV2_BOUNDS(Num) lav2_kernel(const Lav2Args<Num, IterT> A) {
 
         if (live) {
             const size_t cell = (size_t)Y * A.pitch + X;
-            A.out[cell] = iter;
-            if (A.sink) A.sink[cell] = iter; // 8 lanes per row: one 32-byte posted write
+            if constexpr (Frames) {
+                // this tile's ticket is cursor.cur - 1 (next_tile hands out `cur` and advances it): the frame is derived
+                // again here rather than held across the tile, which would cost HDRx32 a register beyond its bound of 64
+                A.frames[(cursor.cur - 1) / n_tiles].out[cell] = iter;
+            } else {
+                A.out[cell] = iter;
+                if (A.sink) A.sink[cell] = iter; // 8 lanes per row: one 32-byte posted write
+            }
         }
 #ifdef FS_TILE_TIMING
         if (lane == 0 && fs_tile_times) {

@@ -1983,6 +1983,30 @@ fsh_view *fsh_view_create(const char *minX, const char *minY, const char *maxX, 
     return v;
 }
 
+// A frame of a zoom sequence around v's centre: the same cx, cy, precision and size, bounds = centre -/+ v's half-extents
+// times `scale` (a decimal string; > 1 zooms out).  The offsets are formed at extra precision, so scale "1" gives v's
+// bounds bit for bit and scale "2" exactly twice its extents.  Frames of one sequence share v's reference orbit.
+fsh_view *fsh_view_zoom(const fsh_view *v, const char *scale) {
+    const unsigned long prec = v->prec, wide = v->prec + 128;
+    Mpf s(wide), d(wide), t(wide);
+    if (fs_mpf_set_str(s.v, scale, 10) || fs_mpf_sgn(s.v) <= 0) return nullptr;
+    fsh_view *z = new fsh_view(prec);
+    z->w = v->w; z->h = v->h; z->aa = v->aa;
+    fs_mpf_set(z->cx.v, v->cx.v);
+    fs_mpf_set(z->cy.v, v->cy.v);
+    auto side = [&](Mpf &dst, const Mpf &bound, const Mpf &centre) { // dst = centre + (bound - centre) * scale
+        fs_mpf_sub(d.v, bound.v, centre.v);
+        fs_mpf_mul(t.v, d.v, s.v);
+        fs_mpf_add(t.v, centre.v, t.v);
+        fs_mpf_set(dst.v, t.v);
+    };
+    side(z->minX, v->minX, v->cx);
+    side(z->maxX, v->maxX, v->cx);
+    side(z->minY, v->minY, v->cy);
+    side(z->maxY, v->maxY, v->cy);
+    return z;
+}
+
 void fsh_view_destroy(fsh_view *v) { delete v; }
 uint32_t fsh_view_precision_bits(const fsh_view *v) { return (uint32_t)v->prec; }
 

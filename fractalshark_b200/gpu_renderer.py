@@ -104,6 +104,23 @@ class GPURenderer:
             self._h, int(algorithm), int(t.numeric), int(t.mode), int(t.pextras), _buf(coords["cx"]), _buf(coords["cy"]),
             _buf(coords["dx"]), _buf(coords["dy"]), _buf(coords["center_x"]), _buf(coords["center_y"]), n_iterations))
 
+    def RenderPerturbLAv2Frames(self, algorithm: RenderAlgorithm, coords_list, n_iterations: int) -> int:
+        """A zoom batch (``fs_render_perturb_lav2_frames``): one frame per entry of ``coords_list`` (dicts as
+        ``View.coords`` returns, 1 to 64 of them), all with the uploaded orbit and LA table, in one launch.  Frame 0
+        lands in the iteration buffer; ``SelectFrame(k)`` picks the frame ``RenderCurrent`` returns."""
+        t = traits(algorithm)
+        coords_list = list(coords_list)
+
+        def cat(key):
+            return _buf(b"".join(c[key] for c in coords_list)) if coords_list else None
+        return int(self._lib.fs_render_perturb_lav2_frames(
+            self._h, int(algorithm), int(t.numeric), int(t.mode), int(t.pextras), len(coords_list), cat("cx"), cat("cy"),
+            cat("dx"), cat("dy"), cat("center_x"), cat("center_y"), n_iterations))
+
+    def SelectFrame(self, k: int) -> int:
+        """Frame of the last render that ``RenderCurrent`` / ``RenderCurrentShard`` / ``DeviceIterBuffer`` read."""
+        return int(self._lib.fs_select_frame(self._h, k))
+
     def RenderPerturbBLA(self, algorithm: RenderAlgorithm, perturb, blas, coords: dict, n_iterations: int,
                          iteration_precision: int = 1) -> int:
         """``perturb`` is a :class:`host_inputs.Orbit`, ``blas`` a :class:`host_inputs.BlaTable`; both are uploaded

@@ -35,6 +35,18 @@ class View:
             self._lib.fsh_view_destroy(self._h)
             self._h = None
 
+    def zoomed(self, scale: str) -> "View":
+        """A frame of a zoom sequence around this view's centre: the same centre, precision, size and antialiasing,
+        bounds = centre -/+ this view's half-extents x ``scale`` (a decimal string; "2" shows twice the extent).  Such
+        frames share this view's reference orbit and LA table (``GPURenderer.RenderPerturbLAv2Frames``)."""
+        h = self._lib.fsh_view_zoom(self._h, scale.encode())
+        if not h:
+            raise ValueError(f"bad zoom scale {scale!r}")
+        z = View.__new__(View)
+        z._lib, z._h = self._lib, h
+        z.width, z.height, z.antialiasing = self.width, self.height, self.antialiasing
+        return z
+
     @property
     def precision_bits(self) -> int:
         return int(self._lib.fsh_view_precision_bits(self._h))

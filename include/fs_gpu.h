@@ -139,6 +139,27 @@ uint32_t fs_render_perturb_lav2(fs_renderer *r, uint32_t algorithm, int32_t nume
                                 const void *cx, const void *cy, const void *dx, const void *dy, const void *center_x,
                                 const void *center_y, uint64_t n_iterations);
 
+/* Zoom batch (no reference counterpart): n_frames frames of the uploaded orbit and LA table in one launch -- the frames
+ * of a zoom sequence share the view centre, hence the reference orbit.  Each coordinate pointer holds n_frames PODs of
+ * `numeric` back to back (frame f at byte offset f * sizeof(POD)); algorithm, numeric, mode, pextras and n_iterations
+ * are the same for every frame.  Enqueue only; the arrays are read before the call returns.  fs_set_shard applies to
+ * every frame; the frames of a device group are sharded over its members like a single frame.  Frame 0 renders into the
+ * iteration buffer, frames 1..n_frames-1 into a frame stack the renderer grows on demand; fs_select_frame picks the one
+ * the result calls read.  The batch always runs the fused LAv2 tile kernel: fs_set_split_at, fs_set_pool_kernel and the
+ * small-shard probe order do not apply (they change scheduling, never results).  The result sink is not written and is
+ * left unfilled, so the next fs_render_current copies.  fs_last_render_ms and the step counters cover the whole batch.
+ * n_frames outside [1, FS_MAX_FRAMES], a NULL renderer or a NULL dx/dy/center pointer: FS_ERROR_UNSUPPORTED, before any
+ * CUDA call.  Frames that differ in scale need nothing extra: the AT shortcut's usability test is per pixel. */
+#define FS_MAX_FRAMES 64
+uint32_t fs_render_perturb_lav2_frames(fs_renderer *r, uint32_t algorithm, int32_t numeric, int32_t mode, int32_t pextras,
+                                       uint32_t n_frames, const void *cx, const void *cy, const void *dx, const void *dy,
+                                       const void *center_x, const void *center_y, uint64_t n_iterations);
+/* Subsequent fs_render_current / fs_render_current_shard / fs_device_iter_buffer read frame k of the last render
+ * (colours and Min/Max/Sum are computed from that frame).  Every render call selects frame 0; a single-frame render
+ * counts as one frame.  k >= the last render's frame count (any k before the first render): FS_ERROR_UNSUPPORTED and
+ * the selection is unchanged.  A device group selects the frame on every member. */
+uint32_t fs_select_frame(fs_renderer *r, uint32_t k);
+
 /* GPURenderer::RenderPerturbBLA<IterType,T>  GPU_Render.h:51-77 */
 uint32_t fs_render_perturb_bla(fs_renderer *r, uint32_t algorithm, int32_t numeric, const fs_orbit *results,
                                const fs_blas *blas, const void *cx, const void *cy, const void *dx, const void *dy,
