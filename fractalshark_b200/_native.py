@@ -52,6 +52,7 @@ GPU_SYMBOLS = {
     "fs_render_perturb_lav2": (_U32, [_V, _U32, _I32, _I32, _I32, _V, _V, _V, _V, _V, _V, _U64]),
     "fs_render_perturb_lav2_frames": (_U32, [_V, _U32, _I32, _I32, _I32, _U32, _V, _V, _V, _V, _V, _V, _U64]),
     "fs_select_frame": (_U32, [_V, _U32]),
+    "fs_render_perturb_lav2_expmap": (_U32, [_V, _U32, _I32, _I32, _I32, _V, _V, _V, _U64]),
     "fs_render_perturb_bla": (_U32, [_V, _U32, _I32, C.POINTER(FsOrbit), C.POINTER(FsBlas), _V, _V, _V, _V, _V, _V,
                                      _U64, _I32]),
     "fs_render_perturb_bla_scaled": (_U32, [_V, _U32, _I32, C.POINTER(FsOrbit), C.POINTER(FsOrbit), _V, _V, _V, _V,
@@ -89,6 +90,8 @@ HOST_SYMBOLS = {
     "fsh_view_destroy": (None, [_V]),
     "fsh_view_precision_bits": (_U32, [_V]),
     "fsh_view_coords": (_I32, [_V, _I32, _V, _V, _V, _V, _V, _V]),
+    "fsh_view_expmap": (_I32, [_V, _I32, _U32, _V, _V, _V, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+    "fsh_selftest_numeric_op": (_I32, [_U32, _V, _V, _V, _U64]),
     "fsh_orbit_compute": (_V, [_V, _I32, _U64, _I32]),
     "fsh_orbit_with_bad": (_V, [_V, _I32]),
     "fsh_orbit_compress": (_V, [_V, _I32]),

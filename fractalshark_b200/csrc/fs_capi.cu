@@ -153,6 +153,7 @@ struct fs_renderer {
     uint32_t stack_frames = 0;
     uint32_t n_frames = 0, selected = 0; // n_frames = 0: nothing rendered since the buffers were allocated
     DeviceBlob frame_recs;               // the batch's Lav2Frame records
+    DeviceBlob expmap_tables;            // fs_render_perturb_lav2_expmap: radius[height], dir_x[width], dir_y[width]
 };
 
 namespace {
@@ -225,6 +226,7 @@ void reset_buffers(fs_renderer *r) {
     drop_sink(r);
     free_blob(r, r->at_state);
     free_blob(r, r->frame_recs);
+    free_blob(r, r->expmap_tables);
     if (r->frame_stack) cudaFreeAsync(r->frame_stack, r->compute);
     r->frame_stack = nullptr;
     r->stack_frames = 0;
@@ -714,7 +716,7 @@ uint32_t launch_lav2(fs_renderer *r, int mode, const void *dx, const void *dy, c
     return end_render(r);
 }
 
-// A zoom batch: n_frames frames of r's orbit and tables in one launch of lav2_kernel<..., Frames = true>.  `dx` ... `cy`
+// A zoom batch: n_frames frames of r's orbit and tables in one launch of lav2_kernel<..., Lav2Layout::Frames>.  `dx` ... `cy`
 // hold n_frames PODs each.  The batch always runs the fused tile kernel: the split-AT, lane-refill and probe-order
 // switches of launch_lav2 only change how a single frame is scheduled, never its cells, so a batch ignores them.
 template <class Num, class IterT>
@@ -767,14 +769,62 @@ uint32_t launch_lav2_frames(fs_renderer *r, int mode, uint32_t n_frames, const v
     r->n_frames = n_frames;
     const bool count = r->count_steps;
 #define FS_LAUNCH_FRAMES(MODE)                                                                                         \
-    if (count) { auto k = lav2_kernel<Num, IterT, MODE, true, AtPhase::Fused, true>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); } \
-    else { auto k = lav2_kernel<Num, IterT, MODE, false, AtPhase::Fused, true>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); }
+    if (count) { auto k = lav2_kernel<Num, IterT, MODE, true, AtPhase::Fused, Lav2Layout::Frames>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); } \
+    else { auto k = lav2_kernel<Num, IterT, MODE, false, AtPhase::Fused, Lav2Layout::Frames>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); }
     switch (mode) {
     case FS_LAV2_FULL: FS_LAUNCH_FRAMES(Lav2Mode::Full) break;
     case FS_LAV2_PO: FS_LAUNCH_FRAMES(Lav2Mode::PO) break;
     default: FS_LAUNCH_FRAMES(Lav2Mode::LAO) break;
     }
 #undef FS_LAUNCH_FRAMES
+    return end_render(r);
+}
+
+// An exponential map: one frame of lav2_kernel<..., Lav2Layout::ExpMap>, pixel (X, Y) at dc = expmap_dc(radius[Y],
+// dir_x[X], dir_y[X]).  The tables are copied into renderer-owned device memory before the call returns.  Like a zoom
+// batch it always runs the fused tile kernel (the split-AT, lane-refill and probe-order switches change scheduling, never
+// cells); otherwise it is a single-frame render: frame 0, the result sink, the shard rule.
+template <class Num, class IterT>
+uint32_t launch_lav2_expmap(fs_renderer *r, int mode, const void *radius, const void *dir_x, const void *dir_y,
+                            uint64_t n_iter) {
+    using Real = typename Num::Real;
+    const uint64_t bands = ((r->height + 3) / 4 + r->shard_count - 1 - r->shard_index) / r->shard_count;
+    if ((r->width + 7) / 8 * bands >= (1ull << 31)) return FS_ERROR_UNSUPPORTED; // tickets are 32-bit
+    const size_t h_bytes = (size_t)r->height * sizeof(Real), w_bytes = (size_t)r->width * sizeof(Real);
+    const size_t need = h_bytes + 2 * w_bytes;
+    if (r->expmap_tables.bytes < need) {
+        free_blob(r, r->expmap_tables);
+        cudaError_t err = cudaMallocAsync(&r->expmap_tables.ptr, need, r->compute);
+        if (err != cudaSuccess) return err;
+        r->expmap_tables.bytes = need;
+    }
+    // one staging copy in pageable memory: cudaMemcpyAsync has consumed it when it returns, whatever memory the caller's
+    // tables are in, so the caller may reuse them at once
+    std::vector<unsigned char> host(need);
+    memcpy(host.data(), radius, h_bytes);
+    memcpy(host.data() + h_bytes, dir_x, w_bytes);
+    memcpy(host.data() + h_bytes + w_bytes, dir_y, w_bytes);
+    cudaError_t err = cudaMemcpyAsync(r->expmap_tables.ptr, host.data(), need, cudaMemcpyHostToDevice, r->compute);
+    if (err != cudaSuccess) return err;
+    bool have_la = false;
+    Real unused;
+    memset(&unused, 0, sizeof(unused));
+    Lav2Args<Num, IterT> A = lav2_args<Num, IterT>(r, &unused, &unused, &unused, &unused, n_iter, have_la);
+    const unsigned char *tables = static_cast<const unsigned char *>(r->expmap_tables.ptr);
+    A.exp_radius = reinterpret_cast<const Real *>(tables);
+    A.exp_dir_x = reinterpret_cast<const Real *>(tables + h_bytes);
+    A.exp_dir_y = reinterpret_cast<const Real *>(tables + h_bytes + w_bytes);
+    begin_render(r, true);
+    const bool count = r->count_steps;
+#define FS_LAUNCH_EXPMAP(MODE)                                                                                         \
+    if (count) { auto k = lav2_kernel<Num, IterT, MODE, true, AtPhase::Fused, Lav2Layout::ExpMap>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); } \
+    else { auto k = lav2_kernel<Num, IterT, MODE, false, AtPhase::Fused, Lav2Layout::ExpMap>; k<<<lav2_grid(r, k), 256, 0, r->compute>>>(A); }
+    switch (mode) {
+    case FS_LAV2_FULL: FS_LAUNCH_EXPMAP(Lav2Mode::Full) break;
+    case FS_LAV2_PO: FS_LAUNCH_EXPMAP(Lav2Mode::PO) break;
+    default: FS_LAUNCH_EXPMAP(Lav2Mode::LAO) break;
+    }
+#undef FS_LAUNCH_EXPMAP
     return end_render(r);
 }
 
@@ -1179,6 +1229,20 @@ __global__ void numeric_op_kernel(uint32_t op, const void *a_, const void *b_, v
         }
         break;
     }
+    case 86: case 87: case 88: case 89: case 90: case 91: { // exp-map pixel -> dc (fs_num.cuh expmap_dc), 32-byte elements
+        const size_t at = (size_t)kExpmapRecordBytes * i;
+        const unsigned char *a = static_cast<const unsigned char *>(a_) + at, *b = static_cast<const unsigned char *>(b_) + at;
+        unsigned char *o = static_cast<unsigned char *>(out_) + at;
+        switch (op) {
+        case 86: expmap_selftest<NumPlain<float>>(a, b, o); break;
+        case 87: expmap_selftest<NumPlain<double>>(a, b, o); break;
+        case 88: expmap_selftest<NumHdr<float>>(a, b, o); break;
+        case 89: expmap_selftest<NumHdr<double>>(a, b, o); break;
+        case 90: expmap_selftest<Num2x32>(a, b, o); break;
+        default: expmap_selftest<NumHdr2x32>(a, b, o); break;
+        }
+        break;
+    }
     case 30: static_cast<dd64 *>(out_)[i] = dd_add(qa[i], qb[i]); break;
     case 31: static_cast<dd64 *>(out_)[i] = dd_sub(qa[i], qb[i]); break;
     case 32: static_cast<dd64 *>(out_)[i] = dd_mul(qa[i], qb[i]); break;
@@ -1203,6 +1267,7 @@ uint32_t numeric_op_elem_bytes(uint32_t op) {
     if (op >= 60 && op <= 67) return 32;
     if (op >= 70 && op <= 77) return 16;
     if (op >= 80 && op <= 85) return kPerturbRecordBytes;
+    if (op >= 86 && op <= 91) return kExpmapRecordBytes;
     return 0;
 }
 } // namespace
@@ -1549,6 +1614,24 @@ uint32_t fs_render_perturb_lav2_frames(fs_renderer *r, uint32_t algorithm, int32
     if (pextras != FS_PEXTRAS_DISABLE && pextras != FS_PEXTRAS_SIMPLE_COMPRESSION) return FS_ERROR_UNSUPPORTED;
     return dispatch_num_iter(numeric, r->iter_bytes, [&](auto num, auto it) -> uint32_t {
         return launch_lav2_frames<decltype(num), decltype(it)>(r, mode, n_frames, dx, dy, center_x, center_y, n_iterations);
+    });
+}
+
+uint32_t fs_render_perturb_lav2_expmap(fs_renderer *r, uint32_t algorithm, int32_t numeric, int32_t mode, int32_t pextras,
+                                       const void *radius, const void *dir_x, const void *dir_y, uint64_t n_iterations) {
+    if (!r || !radius || !dir_x || !dir_y) return FS_ERROR_UNSUPPORTED;
+    if (mode != FS_LAV2_FULL && mode != FS_LAV2_PO && mode != FS_LAV2_LAO) return FS_ERROR_UNSUPPORTED;
+    if (is_group(r))
+        return each_member(r, [&](fs_renderer *m) {
+            return fs_render_perturb_lav2_expmap(m, algorithm, numeric, mode, pextras, radius, dir_x, dir_y, n_iterations);
+        });
+    (void)algorithm;
+    if (!memory_initialized(r)) return FS_ERROR_UNSUPPORTED; // the tables' sizes are the initialized frame's
+    DeviceGuard g(r->device);
+    if (!r->orbit1.valid || r->orbit1.numeric != numeric || r->orbit1.pextras != pextras) return FS_ERROR_6_NO_ORBIT;
+    if (pextras != FS_PEXTRAS_DISABLE && pextras != FS_PEXTRAS_SIMPLE_COMPRESSION) return FS_ERROR_UNSUPPORTED;
+    return dispatch_num_iter(numeric, r->iter_bytes, [&](auto num, auto it) -> uint32_t {
+        return launch_lav2_expmap<decltype(num), decltype(it)>(r, mode, radius, dir_x, dir_y, n_iterations);
     });
 }
 

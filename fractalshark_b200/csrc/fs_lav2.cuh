@@ -139,9 +139,16 @@ template <class Num, class IterT> struct Lav2Args {
     const unsigned int *order;        // optional: queue position -> tile ticket (lav2_probe_kernel: expensive tiles first)
     int at_cycle;                     // 1: cycle detection in the AT shortcut (CycleWatch), 0: every pass is executed
     IterT *sink;                      // optional mapped host copy of `out` (fs_set_result_sink): finished pixels stream out over PCIe
-    const Lav2Frame<Num, IterT> *frames; // lav2_kernel<..., Frames = true>: n_frames records; dx, dy, centerX, centerY, out unused
+    const Lav2Frame<Num, IterT> *frames; // Lav2Layout::Frames: n_frames records; dx, dy, centerX, centerY, out unused
     unsigned int n_frames;
+    // Lav2Layout::ExpMap: height radii and width directions (expmap_dc); dx, dy, centerX, centerY unused
+    const typename Num::Real *exp_radius, *exp_dir_x, *exp_dir_y;
 };
+
+// How lav2_kernel maps pixels to dc and where it stores them.  Rect: one frame, dc = delta_x / delta_y of the linear map
+// (fs_render_perturb_lav2).  Frames: a zoom batch of linear maps (fs_render_perturb_lav2_frames).  ExpMap: one frame of an
+// exponential map, dc = expmap_dc of its tables (fs_render_perturb_lav2_expmap); otherwise the Rect code.
+enum class Lav2Layout : int { Rect = 0, Frames = 1, ExpMap = 2 };
 
 // How a launch treats the AT shortcut.  Fused = one launch does everything (the reference's structure).  On deep views
 // the AT loop is most of the frame and perfectly regular (every interior pixel runs n/StepLength passes) while what
@@ -650,16 +657,21 @@ FS_D void lav2_stages_v2(const Lav2Args<NumHdr<float>, uint32_t> &A, const HdrC<
     }
 }
 
-// Frames = true renders a zoom batch: A.n_frames frames that share the orbit and the tables, each with its own pixel
+// Layout Frames renders a zoom batch: A.n_frames frames that share the orbit and the tables, each with its own pixel
 // spacing, centre offset and iteration buffer (A.frames).  The queue hands out n_frames x n_tiles tickets, frame-major,
 // so the SMs that finish frame k's cheap tiles pick up frame k + 1's while frame k's expensive tiles still run: only the
 // last frame's tail is left at the end of the launch.  Tiles of every frame keep the centre-out order and the shard rule.
 // No result sink, no probe order.
-template <class Num, class IterT, Lav2Mode Mode, bool Count, AtPhase Phase = AtPhase::Fused, bool Frames = false>
+// Layout ExpMap renders an exponential map: pixel (X, Y) takes dc = expmap_dc(radius[Y], dir_x[X], dir_y[X]) in place of
+// the linear map's delta_x / delta_y; everything else -- queue, shard rule, store, result sink, step counters -- is the
+// single-frame code.  No probe order (lav2_probe_kernel assumes the linear map).
+template <class Num, class IterT, Lav2Mode Mode, bool Count, AtPhase Phase = AtPhase::Fused,
+          Lav2Layout Layout = Lav2Layout::Rect>
 __global__ void FS_LAV2_BOUNDS(Num) lav2_kernel(const Lav2Args<Num, IterT> A) {
     using Real = typename Num::Real;
     using Cplx = typename Num::Cplx;
-    static_assert(!Frames || Phase == AtPhase::Fused, "zoom batches run the fused kernel");
+    constexpr bool Frames = Layout == Lav2Layout::Frames;
+    static_assert(Layout == Lav2Layout::Rect || Phase == AtPhase::Fused, "zoom batches and exp maps run the fused kernel");
 
     const int lane = threadIdx.x & 31;
     const int tiles_x = (A.width + 7) >> 3;
@@ -689,7 +701,7 @@ __global__ void FS_LAV2_BOUNDS(Num) lav2_kernel(const Lav2Args<Num, IterT> A) {
         unsigned long long fs_g0;
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(fs_g0));
 #endif
-        if (!Frames && A.order) {
+        if (Layout == Lav2Layout::Rect && A.order) {
             // two lists filled by lav2_probe_kernel, each in ticket (centre-out) order: expensive tiles, then the rest
             const unsigned int n_first = *(const volatile unsigned int *)(A.order + 2 * (size_t)n_tiles);
             tile = tile < n_first ? __ldg(A.order + tile) : __ldg(A.order + n_tiles + (tile - n_first));
@@ -703,9 +715,16 @@ __global__ void FS_LAV2_BOUNDS(Num) lav2_kernel(const Lav2Args<Num, IterT> A) {
 
         IterT iter = 0;
         IterT RefIteration = 0;
-        // LAKernel.cuh:41-42 (no reduction of the deltas here)
-        const Real dcX = Num::delta_x(fdx, X, fcx);
-        const Real dcY = Num::delta_y(fdy, Y, fcy);
+        Real dcX, dcY;
+        if constexpr (Layout == Lav2Layout::ExpMap) {
+            // lanes outside the image read the last row / column: their cells are never stored
+            const int tx = X < A.width ? X : A.width - 1, ty = Y < A.height ? Y : A.height - 1;
+            expmap_dc<Num>(A.exp_radius[ty], A.exp_dir_x[tx], A.exp_dir_y[tx], dcX, dcY);
+        } else {
+            // LAKernel.cuh:41-42 (no reduction of the deltas here)
+            dcX = Num::delta_x(fdx, X, fcx);
+            dcY = Num::delta_y(fdy, Y, fcy);
+        }
         const Cplx dc = Num::c_make(dcX, dcY);
         Cplx dz = Num::c_zero();
 

@@ -147,4 +147,29 @@ template <class Num> FS_HD void perturb_selftest(const unsigned char *in, unsign
     for (int k = 0; k < 6; k++) memcpy(out + 16 * k, &r[k], sizeof(Real));
 }
 
+// Pixel -> dc of an exponential map (fs_render_perturb_lav2_expmap): pixel (X, Y) lies at radius rho = radius[Y] from the
+// reference point in direction (ux, uy) = (dir_x[X], dir_y[X]), and dc = (rho * ux, rho * uy) with the type's own multiply.
+// The LAv2 kernel and the self-test ops 86-91 both call this function.
+template <class Num>
+FS_HD void expmap_dc(typename Num::Real rho, typename Num::Real ux, typename Num::Real uy, typename Num::Real &dcX,
+                     typename Num::Real &dcY) {
+    dcX = mul(rho, ux);
+    dcY = mul(rho, uy);
+}
+
+// Self-test of expmap_dc (fs_selftest_numeric_op 86-91, host: fsh_selftest_numeric_op 86-89): elements of two 16-byte
+// cells, each cell one Real in its in-memory layout.  a = {rho, unused}, b = {ux, uy}, out = {dcX, dcY}.
+constexpr int kExpmapRecordBytes = 32;
+template <class Num> FS_HD void expmap_selftest(const unsigned char *a, const unsigned char *b, unsigned char *out) {
+    using Real = typename Num::Real;
+    static_assert(sizeof(Real) <= 16, "one cell per number");
+    Real rho, ux, uy, r[2];
+    memcpy(&rho, a, sizeof(Real));
+    memcpy(&ux, b, sizeof(Real));
+    memcpy(&uy, b + 16, sizeof(Real));
+    expmap_dc<Num>(rho, ux, uy, r[0], r[1]);
+    for (int k = 0; k < kExpmapRecordBytes; k++) out[k] = 0;
+    for (int k = 0; k < 2; k++) memcpy(out + 16 * k, &r[k], sizeof(Real));
+}
+
 } // namespace fs

@@ -26,6 +26,7 @@ void __gmpf_mul(fs_mpf_struct *, const fs_mpf_struct *, const fs_mpf_struct *);
 void __gmpf_div(fs_mpf_struct *, const fs_mpf_struct *, const fs_mpf_struct *);
 void __gmpf_div_ui(fs_mpf_struct *, const fs_mpf_struct *, unsigned long);
 void __gmpf_mul_2exp(fs_mpf_struct *, const fs_mpf_struct *, unsigned long);
+void __gmpf_div_2exp(fs_mpf_struct *, const fs_mpf_struct *, unsigned long);
 double __gmpf_get_d(const fs_mpf_struct *);
 double __gmpf_get_d_2exp(long *, const fs_mpf_struct *);
 int __gmpf_cmp(const fs_mpf_struct *, const fs_mpf_struct *);
@@ -43,6 +44,7 @@ int __gmpf_cmp(const fs_mpf_struct *, const fs_mpf_struct *);
 #define fs_mpf_div __gmpf_div
 #define fs_mpf_div_ui __gmpf_div_ui
 #define fs_mpf_mul_2exp __gmpf_mul_2exp
+#define fs_mpf_div_2exp __gmpf_div_2exp
 #define fs_mpf_get_d __gmpf_get_d
 #define fs_mpf_get_d_2exp __gmpf_get_d_2exp
 #define fs_mpf_cmp __gmpf_cmp

@@ -28,6 +28,7 @@
 #include <unistd.h>
 
 #include "../fs_types.cuh"
+#include "../fs_num.cuh"
 #include "fs_gmp_min.h"
 
 using namespace fs;
@@ -1935,6 +1936,27 @@ template <class N> void fill_coord(const fs_mpf_struct *f, void *dst) {
     memcpy(dst, &v, sizeof(v));
 }
 
+// FillCoord for the 2x32 types (Fractal.cpp:1813-1826): CudaDblflt(double(src)); HDRFloat<CudaDblflt>(src)
+// splits the mpf mantissa into head/tail without renormalising and does NOT reduce
+void fill_df(const fs_mpf_struct *f, void *dst, bool hdr) {
+    if (!dst) return;
+    if (!hdr) {
+        const df32 v = h_df_from_double(fs_mpf_get_d(f));
+        memcpy(dst, &v, sizeof(v));
+    } else {
+        Hdr<df32> v;
+        if (fs_mpf_sgn(f) == 0) { v.m.head = 0; v.m.tail = 0; v.e = MIN_BIG; }
+        else {
+            long e = 0;
+            const double m = fs_mpf_get_d_2exp(&e, f);
+            v.m.head = (float)m;
+            v.m.tail = (float)(m - (double)v.m.head);
+            v.e = (int32_t)e;
+        }
+        memcpy(dst, &v, sizeof(v));
+    }
+}
+
 } // namespace
 
 extern "C" {
@@ -2026,26 +2048,6 @@ int32_t fsh_view_coords(const fsh_view *v, int32_t numeric, void *cx, void *cy, 
 #define FSH_FILL(N)                                                                                                    \
     fill_coord<N>(v->minX.v, cx); fill_coord<N>(v->minY.v, cy); fill_coord<N>(ddx.v, dx); fill_coord<N>(ddy.v, dy);   \
     fill_coord<N>(cenx.v, center_x); fill_coord<N>(ceny.v, center_y); return 0;
-    // FillCoord for the 2x32 types (Fractal.cpp:1813-1826): CudaDblflt(double(src)); HDRFloat<CudaDblflt>(src)
-    // splits the mpf mantissa into head/tail without renormalising and does NOT reduce
-    auto fill_df = [&](const fs_mpf_struct *f, void *dst, bool hdr) {
-        if (!dst) return;
-        if (!hdr) {
-            const df32 v = h_df_from_double(fs_mpf_get_d(f));
-            memcpy(dst, &v, sizeof(v));
-        } else {
-            Hdr<df32> v;
-            if (fs_mpf_sgn(f) == 0) { v.m.head = 0; v.m.tail = 0; v.e = MIN_BIG; }
-            else {
-                long e = 0;
-                const double m = fs_mpf_get_d_2exp(&e, f);
-                v.m.head = (float)m;
-                v.m.tail = (float)(m - (double)v.m.head);
-                v.e = (int32_t)e;
-            }
-            memcpy(dst, &v, sizeof(v));
-        }
-    };
     // FillCoord for the direct kernels' split types (Fractal.cpp:1752-1779, 1805-1810): limb k is the
     // conversion of what is left after subtracting limbs 0..k-1 in full precision
     auto fill_split = [&](const fs_mpf_struct *f, void *dst, int limbs, bool as_float) {
@@ -2088,6 +2090,94 @@ int32_t fsh_view_coords(const fsh_view *v, int32_t numeric, void *cx, void *cy, 
     default: return -1;
     }
 #undef FSH_FILL
+}
+
+// Tables of an exponential map around v's centre (fs_render_perturb_lav2_expmap), W = v's super-sampled width:
+//   dir_x[X] + i dir_y[X] = exp(i theta_X), theta_X = 2 pi (X + 1/2) / W  (W PODs each; counter-clockwise, imaginary up)
+//   radius[Y] = radius0 * exp(-2 pi Y / W), radius0 = v's half-diagonal * exp(-pi / W)  (`rows` PODs; row 0 outermost)
+// so pixels are square in the plane at every depth and v's corners lie on the outer edge of row 0's ring.  Every POD is
+// converted from an mpf as the view's coordinates are (fill_coord / fill_df); plain types underflow where they do.  The
+// radii are worked in log2 -- an integer exponent plus a double fraction per row -- so rows 2^-380000 deep keep every
+// fraction bit.  *log2_radius0 and *log2_row_step (-2 pi / (W ln 2)) may be NULL.  Returns 0, or -1 for an unknown
+// numeric, an empty view or a NULL table.
+int32_t fsh_view_expmap(const fsh_view *v, int32_t numeric, uint32_t rows, void *radius, void *dir_x, void *dir_y,
+                        double *log2_radius0, double *log2_row_step) {
+    const uint32_t W = v->w * v->aa;
+    size_t pod = 0;
+    switch (numeric) {
+    case NUM_F32: pod = sizeof(float); break;
+    case NUM_F64: pod = sizeof(double); break;
+    case NUM_2X32: pod = sizeof(df32); break;
+    case NUM_HDR32: pod = sizeof(Hdr<float>); break;
+    case NUM_HDR64: pod = sizeof(Hdr<double>); break;
+    case NUM_HDR2X32: pod = sizeof(Hdr<df32>); break;
+    default: return -1;
+    }
+    if (W == 0 || !radius || !dir_x || !dir_y) return -1;
+    auto fill = [&](const fs_mpf_struct *f, void *dst) {
+        switch (numeric) {
+        case NUM_F32: fill_coord<HostPlain<float>>(f, dst); break;
+        case NUM_F64: fill_coord<HostPlain<double>>(f, dst); break;
+        case NUM_HDR32: fill_coord<HostHdr<float>>(f, dst); break;
+        case NUM_HDR64: fill_coord<HostHdr<double>>(f, dst); break;
+        default: fill_df(f, dst, numeric == NUM_HDR2X32); break;
+        }
+    };
+    const unsigned long prec = v->prec;
+    Mpf d2(prec), t(prec), val(prec);
+    // the squared diagonal, m 2^e with m in [0.5, 1): log2(half-diagonal) = (e + log2 m) / 2 - 1
+    fs_mpf_sub(val.v, v->maxX.v, v->minX.v);
+    fs_mpf_mul(d2.v, val.v, val.v);
+    fs_mpf_sub(val.v, v->maxY.v, v->minY.v);
+    fs_mpf_mul(t.v, val.v, val.v);
+    fs_mpf_add(d2.v, d2.v, t.v);
+    if (fs_mpf_sgn(d2.v) == 0) return -1;
+    long e = 0;
+    const double m = fs_mpf_get_d_2exp(&e, d2.v);
+    const long e_half = e >= 0 ? e / 2 : -((1 - e) / 2); // floor(e / 2)
+    const double step = 2.0 * M_PI / ((double)W * M_LN2); // log2 of the ratio of neighbouring radii
+    // log2 radius0 = base + frac, frac in [0, 1)
+    double frac = (double)(e - 2 * e_half) / 2.0 + log2(m) / 2.0 - 1.0 - step / 2.0;
+    const double fl0 = floor(frac);
+    const long base = e_half + (long)fl0;
+    frac -= fl0;
+    for (uint32_t Y = 0; Y < rows; Y++) {
+        const double g = frac - (double)Y * step, gi = floor(g);
+        const long ex = base + (long)gi;
+        fs_mpf_set_d(val.v, exp2(g - gi));
+        if (ex >= 0) fs_mpf_mul_2exp(val.v, val.v, (unsigned long)ex);
+        else fs_mpf_div_2exp(val.v, val.v, (unsigned long)-ex);
+        fill(val.v, static_cast<char *>(radius) + Y * pod);
+    }
+    for (uint32_t X = 0; X < W; X++) {
+        const double theta = 2.0 * M_PI * ((double)X + 0.5) / (double)W;
+        fs_mpf_set_d(val.v, cos(theta));
+        fill(val.v, static_cast<char *>(dir_x) + X * pod);
+        fs_mpf_set_d(val.v, sin(theta));
+        fill(val.v, static_cast<char *>(dir_y) + X * pod);
+    }
+    if (log2_radius0) *log2_radius0 = (double)base + frac;
+    if (log2_row_step) *log2_row_step = -step;
+    return 0;
+}
+
+// The host build of fs_selftest_numeric_op 86-89: expmap_dc (fs_num.cuh) of the f32, f64, HDRx32 and HDRx64 policies on
+// n elements of 32 bytes (a = {radius, -}, b = {dir_x, dir_y}, out = {dcX, dcY}).  -1: not a host op (the 2x32 policies,
+// ops 90-91, are device-only).
+int32_t fsh_selftest_numeric_op(uint32_t op, const void *a, const void *b, void *out, uint64_t n) {
+    if (op < 86 || op > 89) return -1;
+    for (uint64_t i = 0; i < n; i++) {
+        const size_t at = (size_t)kExpmapRecordBytes * i;
+        const unsigned char *pa = static_cast<const unsigned char *>(a) + at, *pb = static_cast<const unsigned char *>(b) + at;
+        unsigned char *po = static_cast<unsigned char *>(out) + at;
+        switch (op) {
+        case 86: expmap_selftest<NumPlain<float>>(pa, pb, po); break;
+        case 87: expmap_selftest<NumPlain<double>>(pa, pb, po); break;
+        case 88: expmap_selftest<NumHdr<float>>(pa, pb, po); break;
+        default: expmap_selftest<NumHdr<double>>(pa, pb, po); break;
+        }
+    }
+    return 0;
 }
 
 fsh_orbit *fsh_orbit_compute(const fsh_view *v, int32_t numeric, uint64_t max_iterations, int32_t periodicity) {

@@ -117,6 +117,15 @@ class GPURenderer:
             self._h, int(algorithm), int(t.numeric), int(t.mode), int(t.pextras), len(coords_list), cat("cx"), cat("cy"),
             cat("dx"), cat("dy"), cat("center_x"), cat("center_y"), n_iterations))
 
+    def RenderPerturbLAv2ExpMap(self, algorithm: RenderAlgorithm, expmap: dict, n_iterations: int) -> int:
+        """An exponential map (``fs_render_perturb_lav2_expmap``) around the uploaded orbit's reference point: ``expmap``
+        is what ``View.exp_map`` returns, with as many radii as the initialized height and as many directions as the
+        width.  One frame; every cell is the cell a single render of its own dc gives."""
+        t = traits(algorithm)
+        return int(self._lib.fs_render_perturb_lav2_expmap(
+            self._h, int(algorithm), int(t.numeric), int(t.mode), int(t.pextras), _buf(expmap["radius"]),
+            _buf(expmap["dir_x"]), _buf(expmap["dir_y"]), n_iterations))
+
     def SelectFrame(self, k: int) -> int:
         """Frame of the last render that ``RenderCurrent`` / ``RenderCurrentShard`` / ``DeviceIterBuffer`` read."""
         return int(self._lib.fs_select_frame(self._h, k))

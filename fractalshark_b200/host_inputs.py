@@ -63,6 +63,23 @@ class View:
             raise ValueError(f"numeric {numeric!r} not supported by the input generator")
         return {k: bytes(b.raw) for k, b in bufs.items()}
 
+    def exp_map(self, numeric: Numeric, rows: int) -> dict:
+        """Tables of an exponential map around this view's centre (``fsh_view_expmap``) for
+        ``GPURenderer.RenderPerturbLAv2ExpMap``, W = the super-sampled width: ``dir_x`` / ``dir_y`` (W PODs of ``numeric``
+        each) = cos / sin of the angle 2 pi (X + 1/2) / W, ``radius`` (``rows`` PODs) = radius0 * exp(-2 pi Y / W) with
+        radius0 = the half-diagonal * exp(-pi / W), row 0 outermost; ``log2_radius0`` and ``log2_row_step`` as floats.
+        A zoom by Z needs W ln Z / (2 pi) rows."""
+        nb = POD_BYTES[Numeric(numeric)]
+        w = self.width * self.antialiasing
+        radius, dir_x, dir_y = C.create_string_buffer(nb * rows), C.create_string_buffer(nb * w), C.create_string_buffer(nb * w)
+        l0, step = C.c_double(), C.c_double()
+        rc = self._lib.fsh_view_expmap(self._h, int(numeric), int(rows), C.cast(radius, C.c_void_p),
+                                       C.cast(dir_x, C.c_void_p), C.cast(dir_y, C.c_void_p), C.byref(l0), C.byref(step))
+        if rc != 0:
+            raise ValueError(f"numeric {numeric!r} not supported by the exp-map builder")
+        return {"radius": bytes(radius.raw), "dir_x": bytes(dir_x.raw), "dir_y": bytes(dir_y.raw),
+                "log2_radius0": l0.value, "log2_row_step": step.value}
+
 
 class Orbit:
     """High-precision reference orbit stored as GPUReferenceIter<T, Disable>[count]."""

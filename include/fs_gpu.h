@@ -160,6 +160,22 @@ uint32_t fs_render_perturb_lav2_frames(fs_renderer *r, uint32_t algorithm, int32
  * the selection is unchanged.  A device group selects the frame on every member. */
 uint32_t fs_select_frame(fs_renderer *r, uint32_t k);
 
+/* Exponential map (no reference counterpart): one frame whose pixel (X, Y) lies at dc = (radius[Y] * dir_x[X],
+ * radius[Y] * dir_y[X]) from the uploaded orbit's reference point, with the multiply of `numeric` (fsh_view_expmap builds
+ * the tables: column X at angle 2 pi (X + 1/2) / W, row Y at radius radius0 * exp(-2 pi (Y + 1/2) / W), so every row is
+ * one ring of a zoom and a zoom by Z takes W ln Z / (2 pi) rows).  radius holds fs_get_height PODs of `numeric`, dir_x and
+ * dir_y fs_get_width PODs each.  Enqueue only; the tables are copied into renderer-owned device memory before the call
+ * returns.  The same numeric / mode / pextras / iteration-width combinations and orbit check as fs_render_perturb_lav2;
+ * the LA table is used where it matches the orbit, as there.  Every cell is the cell a single render of its own dc gives:
+ * the kernel is the single-frame fused tile kernel with another pixel -> dc map (fs_set_split_at, fs_set_pool_kernel and
+ * the small-shard probe order do not apply: they change scheduling, never results).  It counts as one frame: frame 0,
+ * result sink, fs_set_shard, device groups, fs_last_render_ms and the step counters as for a single render.  A NULL
+ * renderer or table, a mode other than Full / PO / LAO or memory not initialized: FS_ERROR_UNSUPPORTED, before any CUDA
+ * call. */
+uint32_t fs_render_perturb_lav2_expmap(fs_renderer *r, uint32_t algorithm, int32_t numeric, int32_t mode,
+                                       int32_t pextras, const void *radius, const void *dir_x, const void *dir_y,
+                                       uint64_t n_iterations);
+
 /* GPURenderer::RenderPerturbBLA<IterType,T>  GPU_Render.h:51-77 */
 uint32_t fs_render_perturb_bla(fs_renderer *r, uint32_t algorithm, int32_t numeric, const fs_orbit *results,
                                const fs_blas *blas, const void *cx, const void *cy, const void *dx, const void *dy,
@@ -250,7 +266,9 @@ uint32_t fs_set_pool_kernel(fs_renderer *r, int32_t enable);
  * divide, compareToBothPositiveReduced (result in .exp); 10-14 HDRFloatComplex<float> add, mul, Reduce, chebychevNorm,
  * times HDRFloat; 20-23 dblflt add, sub, mul, sqr; 30-32 dbldbl add, sub, mul; 40 the HDRx32 perturbation step (a = {dX, dY, Zx},
  * b = {Zy, cX, cY}, out = {dX', dY', 0}: 24 B each); 50-56 HDRFloat<double> add, sub, mul, square, Reduce, divide, compare
- * ({double mantissa; int32 exp; int32 pad}, 16 B).  Elements: {float mantissa; int32 exp}
+ * ({double mantissa; int32 exp; int32 pad}, 16 B); 86-91 the exponential map's pixel -> dc (expmap_dc) for f32, f64,
+ * HDRx32, HDRx64, 2x32, HDRx2x32 (32 B elements of two 16 B cells, each one POD of the type: a = {radius, -},
+ * b = {dir_x, dir_y}, out = {dcX, dcY}).  Elements: {float mantissa; int32 exp}
  * (8 B), {float re, im; int32 exp} (12 B), {float head, tail} (8 B), {double head, tail} (16 B).  Reference: HDRFloat.h,
  * HDRFloatComplex.h, dblflt.cuh, dbldbl.cuh (the per-type operator tables SURVEY.md section 8 row a8 lists). */
 uint32_t fs_selftest_numeric_op(int32_t device, uint32_t op, const void *a, const void *b, void *out, uint64_t n);
