@@ -36,8 +36,9 @@ struct alignas(16) Rec {
 static_assert(sizeof(Rec) == 64, "la2::Rec");
 
 struct Out {
-    float dre, dim; int de;  // dz' = newdz*ZCoeff + dc*CCoeff
-    float zre, zim; int ze;  // z = Ref' + dz'
+    float dre, dim;  // dz' = newdz*ZCoeff + dc*CCoeff
+    float zre, zim;  // z = Ref' + dz'
+    int de, ze;      // (the mantissa pairs first: la_step_refused returns them through memory as aligned 8-byte pairs)
     bool unusable, rebase;
 };
 
@@ -83,23 +84,31 @@ FS_HD Rec pack(HdrC<float> Ref, HdrC<float> ZCoeff, HdrC<float> CCoeff, Hdr<floa
 }
 
 // One step; false = refused (nothing may be used).
+// The (re, im) halves of every complex operation run as one packed pair (f32x2: FMUL2 / FFMA2), each half the scalar
+// operation it replaces, on the same operands in the same order.  A complex product
+//     re = fma(ar, br, -(ai*bi))    im = fma(ai, br, ar*bi)
+// is fma2(a, br, mul2(rot(a), bi)) with rot(a) = (-ai, ar): -(ai*bi) == (-ai)*bi bit for bit, the sign of a zero included,
+// and rot() and the broadcasts of br, bi are operand modifiers, not instructions.
 FS_HD bool step(const uint4 q0, const uint4 q1, const uint4 q2, const uint4 q3, float dr, float di, int de, float cr,
                 float ci, int ce, Out &o) {
-    const float rr = u2f(q0.x), ri = u2f(q0.y);
+    const f32x2 dz = f2_make(dr, di);
     const int re2 = (int)q0.z;
     // Prepare: t = 2*Ref + dz
     const int d1 = re2 - de;
     const int fa1 = field(d1), fb1 = field(-d1);
     const float ma1 = pow2f(fa1), mb1 = pow2f(fb1);
-    const float tr = fma_(dr, mb1, rr * ma1), ti = fma_(di, mb1, ri * ma1);
+    float tr, ti;
+    f2_split(f2_fma(dz, f2_bcast(mb1), f2_mul(f2_make(u2f(q0.x), u2f(q0.y)), f2_bcast(ma1))), tr, ti);
     const int te = imax(re2, de);
     bool gap = (uint32_t)(fa1 + fb1 - 128) < 7u;
     // w = dz * t, reduced
-    const float wr = fma_(dr, tr, -(di * ti)), wi = fma_(di, tr, dr * ti);
+    const f32x2 w = f2_fma(dz, f2_bcast(tr), f2_mul(f2_rot(dz), f2_bcast(ti)));
+    float wr, wi;
+    f2_split(w, wr, wi);
     if (!sane(abs_(wr) + abs_(wi))) return false;
     const uint32_t wb = f2u(max_(abs_(wr), abs_(wi)));
     const float sc = u2f(0x7f000000u - (wb & 0x7f800000u));
-    const float nr = wr * sc, ni = wi * sc;
+    const f32x2 n = f2_mul(w, f2_bcast(sc));
     // cheb(newdz) >= LAThreshold on (exponent, mantissa) pairs of reduced positive numbers = one signed 64-bit comparison
     // of exponent * 2^23 + mantissa field; the record carries the threshold in that form (th_key).  wb already holds the
     // larger part's own exponent field, so adding it to (de + te - 127) * 2^23 forms the key and the reduced exponent.
@@ -114,14 +123,15 @@ FS_HD bool step(const uint4 q0, const uint4 q1, const uint4 q2, const uint4 q3, 
     const float ccr = u2f(q2.x), cci = u2f(q2.y);
     // (newdz * ZCoeff is formed from the REDUCED newdz, as the reference does: moving 2^-k out of the product is not exact
     // when the smaller component of an un-reduced w sits in the denormal range -- found by tests/…guards[3])
-    const float pr = fma_(nr, zr, -(ni * zi)), pi = fma_(ni, zr, nr * zi);
-    const float qr = fma_(cr, ccr, -(ci * cci)), qi = fma_(ci, ccr, cr * cci);
+    const f32x2 dc = f2_make(cr, ci);
+    const f32x2 p = f2_fma(n, f2_bcast(zr), f2_mul(f2_rot(n), f2_bcast(zi)));
+    const f32x2 q = f2_fma(dc, f2_bcast(ccr), f2_mul(f2_rot(dc), f2_bcast(cci)));
     const int pe = nwe + (int)q1.z, qe = ce + (int)q2.z;
     const int d2 = pe - qe;
     const int fa2 = field(d2), fb2 = field(-d2);
     const float ma2 = pow2f(fa2), mb2 = pow2f(fb2);
-    o.dre = fma_(qr, mb2, pr * ma2);
-    o.dim = fma_(qi, mb2, pi * ma2);
+    const f32x2 d = f2_fma(q, f2_bcast(mb2), f2_mul(p, f2_bcast(ma2)));
+    f2_split(d, o.dre, o.dim);
     o.de = imax(pe, qe);
     gap = gap || (uint32_t)(fa2 + fb2 - 128) < 7u;
     // getZ: z = Ref' + dz'
@@ -129,8 +139,7 @@ FS_HD bool step(const uint4 q0, const uint4 q1, const uint4 q2, const uint4 q3, 
     const int d3 = ne - o.de;
     const int fa3 = field(d3), fb3 = field(-d3);
     const float ma3 = pow2f(fa3), mb3 = pow2f(fb3);
-    o.zre = fma_(o.dre, mb3, u2f(q3.x) * ma3);
-    o.zim = fma_(o.dim, mb3, u2f(q3.y) * ma3);
+    f2_split(f2_fma(d, f2_bcast(mb3), f2_mul(f2_make(u2f(q3.x), u2f(q3.y)), f2_bcast(ma3))), o.zre, o.zim);
     o.ze = imax(ne, o.de);
     gap = gap || (uint32_t)(fa3 + fb3 - 128) < 7u;
     if (gap || !sane(abs_(o.zre) + abs_(o.zim)) || !sane(abs_(o.dre) + abs_(o.dim))) return false;

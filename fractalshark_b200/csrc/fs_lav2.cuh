@@ -44,9 +44,6 @@
 // run since the save), 0: after every chunk of FS_AT_CHUNK passes (finds it once P * 16 / gcd(P, 16) have).
 #define FS_AT_WATCH_EVERY_PASS 0
 #endif
-#ifndef FS_LA2_EARLY_LOADS
-#define FS_LA2_EARLY_LOADS 0
-#endif
 #ifndef FS_LA2_LDG256
 #define FS_LA2_LDG256 1
 #endif
@@ -604,15 +601,7 @@ FS_D void lav2_stages_v2(const Lav2Args<NumHdr<float>, uint32_t> &A, const HdrC<
         while (iter < A.n_iterations) {
             // getLA  GPU_LAReference.h:271-303
             const uint4 *rp = recs + 4 * (size_t)(LAIndex + j);
-#if FS_LA2_EARLY_LOADS
-            // all four quarters are requested before anything is tested (the compiler otherwise sinks the second one
-            // below the first branch of the step and a trip pays two dependent load latencies)
-            uint4 q0, q1, q2, q3;
-            asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(q0.x), "=r"(q0.y), "=r"(q0.z), "=r"(q0.w) : "l"(rp));
-            asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4+16];" : "=r"(q1.x), "=r"(q1.y), "=r"(q1.z), "=r"(q1.w) : "l"(rp));
-            asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4+32];" : "=r"(q2.x), "=r"(q2.y), "=r"(q2.z), "=r"(q2.w) : "l"(rp));
-            asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4+48];" : "=r"(q3.x), "=r"(q3.y), "=r"(q3.z), "=r"(q3.w) : "l"(rp));
-#elif FS_LA2_LDG256
+#if FS_LA2_LDG256
             // two 256-bit loads (sm_100 LDG.256): half the L1 wavefronts of four 128-bit ones when the lanes of the warp are
             // on different records
             uint4 q0, q1, q2, q3;
@@ -628,19 +617,19 @@ FS_D void lav2_stages_v2(const Lav2Args<NumHdr<float>, uint32_t> &A, const HdrC<
             asm volatile("prefetch.global.L1 [%0];" ::"l"(rp + 4));
             asm volatile("prefetch.global.L1 [%0];" ::"l"(rp + 6));
 #endif
+            // The StepLength test follows the step instead of guarding it: ahead of the step it is the first branch, it reads
+            // only the second load, and the compiler sinks the first load below it -- a trip then waits for two load
+            // latencies in a row.  A step past the iteration limit (a pixel's last LA step, at most once per stage) is
+            // computed and dropped.
             const uint32_t l = q2.w;
             la2::Out o;
-            o.unusable = true;
-            o.rebase = false;
-            if (iter + l <= A.n_iterations) {
-                if (!la2::step(q0, q1, q2, q3, dz.re, dz.im, dz.e, dc.re, dc.im, dc.e, o)) {
-                    // results come back through a local of this branch only: `o` stays in registers
-                    la2::Out slow;
-                    la_step_refused(A.las + (LAIndex + j), dz, dc, slow);
-                    o = slow;
-                }
+            if (!la2::step(q0, q1, q2, q3, dz.re, dz.im, dz.e, dc.re, dc.im, dc.e, o)) {
+                // results come back through a local of this branch only: `o` stays in registers
+                la2::Out slow;
+                la_step_refused(A.las + (LAIndex + j), dz, dc, slow);
+                o = slow;
             }
-            if (o.unusable) {
+            if (o.unusable || iter + l > A.n_iterations) {
                 RefIteration = q3.w;
                 break;
             }

@@ -233,25 +233,72 @@ FS_D bool next_tile(const TileQueue &q, TileCursor &tc, unsigned int n_tiles, un
 #endif
 
 // Packed binary32 pairs (sm_100 FMUL2 / FADD2 / FFMA2): two independent IEEE operations per issued instruction,
-// each lane rounded exactly like its scalar counterpart.  Device only.
-#ifdef __CUDACC__
+// each lane rounded exactly like its scalar counterpart.  The host form is the two scalar operations (CPU checkers).
 struct f32x2 {
-    unsigned long long v;
+    unsigned long long v; // lo = bits 0..31, hi = bits 32..63
 };
-FS_D f32x2 f2_make(float lo, float hi) {
+FS_HD f32x2 f2_make(float lo, float hi) {
     f32x2 r;
+#ifdef __CUDA_ARCH__
     asm("mov.b64 %0, {%1, %2};" : "=l"(r.v) : "f"(lo), "f"(hi));
+#else
+    r.v = (unsigned long long)f2u(lo) | ((unsigned long long)f2u(hi) << 32);
+#endif
     return r;
 }
-FS_D void f2_split(f32x2 a, float &lo, float &hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(a.v)); }
-FS_D f32x2 f2_mul(f32x2 a, f32x2 b) { f32x2 r; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v)); return r; }
-FS_D f32x2 f2_add(f32x2 a, f32x2 b) { f32x2 r; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v)); return r; }
-FS_D f32x2 f2_fma(f32x2 a, f32x2 b, f32x2 c) {
+FS_HD void f2_split(f32x2 a, float &lo, float &hi) {
+#ifdef __CUDA_ARCH__
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(a.v));
+#else
+    lo = u2f((uint32_t)a.v);
+    hi = u2f((uint32_t)(a.v >> 32));
+#endif
+}
+FS_HD f32x2 f2_mul(f32x2 a, f32x2 b) {
+#ifdef __CUDA_ARCH__
+    f32x2 r;
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v));
+    return r;
+#else
+    float al, ah, bl, bh;
+    f2_split(a, al, ah);
+    f2_split(b, bl, bh);
+    return f2_make(al * bl, ah * bh);
+#endif
+}
+FS_HD f32x2 f2_add(f32x2 a, f32x2 b) {
+#ifdef __CUDA_ARCH__
+    f32x2 r;
+    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v));
+    return r;
+#else
+    float al, ah, bl, bh;
+    f2_split(a, al, ah);
+    f2_split(b, bl, bh);
+    return f2_make(al + bl, ah + bh);
+#endif
+}
+FS_HD f32x2 f2_fma(f32x2 a, f32x2 b, f32x2 c) {
+#ifdef __CUDA_ARCH__
     f32x2 r;
     asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r.v) : "l"(a.v), "l"(b.v), "l"(c.v));
     return r;
-}
+#else
+    float al, ah, bl, bh, cl, ch;
+    f2_split(a, al, ah);
+    f2_split(b, bl, bh);
+    f2_split(c, cl, ch);
+    return f2_make(fma_(al, bl, cl), fma_(ah, bh, ch));
 #endif
+}
+// (s, s): ptxas reads it as a broadcast operand (`R.F32`), no move
+FS_HD f32x2 f2_bcast(float s) { return f2_make(s, s); }
+// (lo, hi) -> (-hi, lo), i.e. times i.  An exact sign flip; ptxas folds it into the operand (`-R.F32x2.LO_HI.NP`).
+FS_HD f32x2 f2_rot(f32x2 a) {
+    float lo, hi;
+    f2_split(a, lo, hi);
+    return f2_make(-hi, lo);
+}
 
 // ----------------------------------------------------------------------------------------------
 // Mantissa traits: 2^s multipliers and exponent-field surgery, all integer ALU.
