@@ -233,7 +233,7 @@ FS_HD Mode fast_round(const FastElem *tab, IterT last, IterT n_iterations, const
     const IterT n0 = n;
     const int cnt = (int)(idx - (uint32_t)n0); // steps executed (the last one possibly still needing the exact tests)
     IterT n1 = n0 + (IterT)cnt;
-    bool ok = lo >= kLo, done = false;
+    bool ok = lo >= kLo, done = false, recentre = false;
     if (trig && ok) {
         if (!elem_allows(th, L.k)) {
             ok = false;
@@ -254,11 +254,15 @@ FS_HD Mode fast_round(const FastElem *tab, IterT last, IterT n_iterations, const
                 const float Tx2 = Txs * Txs, Ty2 = Tys * Tys, dx2 = dxs * dxs, dy2 = dys * dys;
                 const float N2 = Tx2 + Ty2, D2 = dx2 + dy2;
                 if (N2 < D2 || n1 >= last) {
-                    // rebase: the next step runs on Z_0
+                    // rebase: the next step runs on Z_0.  T itself is exact once its components are >= kLo; a T the
+                    // next chunk may not start from at this scale (|T| >= kHi, or Z_0 not allowed at k) is committed
+                    // and re-centred below instead of sending the whole chunk back to the float+exponent step
                     const FastElem E0 = load_elem_at(tab, 0);
-                    ok = elem_allows(E0.th, L.k) && fmaxf(fabsf(Tx), fabsf(Ty)) < kHi && fminf(fabsf(Tx), fabsf(Ty)) >= kLo;
+                    const float Tlo = fminf(fabsf(Tx), fabsf(Ty));
+                    ok = Tlo >= kLo;
+                    recentre = !(elem_allows(E0.th, L.k) && fmaxf(fabsf(Tx), fabsf(Ty)) < kHi);
                     wx = Tx; wy = Ty; ax = E0.ax; ay = E0.ay;
-                    lo = fminf(fminf(fabsf(Tx), fabsf(Ty)), lo);
+                    lo = fminf(Tlo, lo);
                     n1 = 0;
                 }
             }
@@ -279,7 +283,7 @@ FS_HD Mode fast_round(const FastElem *tab, IterT last, IterT n_iterations, const
     n = n1;
     L.wx = wx; L.wy = wy; L.ax = ax; L.ay = ay;
     const bool budget = (uint64_t)(n_iterations - iter) >= (uint64_t)kChunk;
-    if (budget && fmaxf(fabsf(wx), fabsf(wy)) < kHi && lo >= kLoWarn) return kFast;
+    if (budget && !recentre && fmaxf(fabsf(wx), fabsf(wy)) < kHi && lo >= kLoWarn) return kFast;
     if (budget && renorm<IterT>(tab, L, c, n)) return kFast;
     leave(L, dxm, dxe, dym, dye);
     return kSlow;
